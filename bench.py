@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our arm (B200)
     python bench.py --impl reference --gpus N --steps K --warmup W   # CPU arm
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR  # also write the last timed solve's outputs
 
 Metric (BASELINE.json / bp5/step-64.cu:458-461): DoFs x CG iterations / second,
 as the reference's "pcg-merged" block measures it: one STEP is one full merged
@@ -52,7 +53,16 @@ def parse():
     ap.add_argument("--no-variants", action="store_true", help="skip the second quadrature")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-cells", type=int, default=0, help="cells per direction of the CPU sample (0 = auto)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed solve of each quadrature returned as DIR/<quadrature>_x.npy (a "
+                         "seeded sample of the solution) and DIR/<quadrature>_solve.npy (iterations, final residual, "
+                         "|x|_2), so that two builds can be compared output for output (one GPU only)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the GPU arm (--impl b200)")
+    return args
 
 
 # --------------------------------------------------------------------------- clocks
@@ -181,8 +191,21 @@ def run_reference(args):
 
 
 # --------------------------------------------------------------------------- GPU arm
-def measure_solver(dc, torch, ctx, stream, op, steps, warmup, sampler=None):
-    """K timed merged-CG solves, device-resident b; returns dict of results."""
+DUMP_SAMPLE = 1 << 21          # solution entries --dump-outputs writes per quadrature: 16 MB in fp64
+
+
+def solution_sample(x):
+    """the whole vector if it is small, else its entries at DUMP_SAMPLE indices drawn with a fixed seed: the same
+    indices for the same mesh on every run and every build"""
+    import numpy as np
+    if x.size <= DUMP_SAMPLE:
+        return x
+    return x[np.sort(np.random.default_rng(0).choice(x.size, DUMP_SAMPLE, replace=False))]
+
+
+def measure_solver(dc, torch, ctx, stream, op, steps, warmup, sampler=None, dump=False):
+    """K timed merged-CG solves, device-resident b; returns dict of results.  dump: also return what the caller of
+    the last timed solve received (under "outputs")."""
     import numpy as np
     n = op.n_owned
     b, x = op.initialize_dof_vector(), op.initialize_dof_vector()
@@ -213,6 +236,11 @@ def measure_solver(dc, torch, ctx, stream, op, steps, warmup, sampler=None):
     launches = ctx.launch_count - launches0
     xnorm = x.l2_norm()
     last_value = control.last_value()
+    outputs = None
+    if dump:
+        # taken here: the profiled pass below solves into the same x
+        outputs = {"x": solution_sample(x.to_host()),
+                   "solve": np.array([control.last_step(), last_value, xnorm], dtype=np.float64)}
     # profiled pass, still under the clock sampler: the same solve with a CUDA event pair around every launch of
     # the dominant kernel (graph replay off), for roofline.achieved; also timed as a whole for comparison
     op.profile(True)
@@ -231,7 +259,7 @@ def measure_solver(dc, torch, ctx, stream, op, steps, warmup, sampler=None):
     clocks = sampler.stop() if sampler else None
     res = dict(secs=secs, its_total=its_total, its_per_step=its_total / steps, n=n, launches=launches,
                kernel_launches=k_launches, kernel_ms=k_ms, bnorm=bnorm, xnorm=xnorm, last_value=last_value,
-               clocks=clocks, prof_secs=prof_secs, prof_its=prof_its)
+               clocks=clocks, prof_secs=prof_secs, prof_its=prof_its, outputs=outputs)
     b.close(); x.close()
     return res
 
@@ -436,6 +464,8 @@ def run_b200(args):
         if world == 1 and args.gpus > 1:
             raise SystemExit("launch N>1 with torch.distributed.run (one rank per GPU)")
     if world > 1:
+        if args.dump_outputs:
+            raise SystemExit("--dump-outputs: one GPU only")
         import bench_multi
         return bench_multi.run(args)
 
@@ -459,13 +489,18 @@ def run_b200(args):
                                                      deformation=1 if args.deformation else 0, eps=args.deformation,
                                                      geometry_mode=geom))
         sampler = ClockSampler(local_rank) if qi == 0 else None
-        r = measure_solver(dc, torch, ctx, stream, op, args.steps, args.warmup, sampler)
+        r = measure_solver(dc, torch, ctx, stream, op, args.steps, args.warmup, sampler, dump=bool(args.dump_outputs))
         bytes_vmult, bytes_cg = op.algorithmic_bytes()
         r["bytes_vmult"], r["bytes_cg"], r["kernel"] = bytes_vmult, bytes_cg, op.kernel_name
         if qi == 0:
             r["e2e"] = measure_e2e(dc, torch, ctx, stream, op, max(1, min(args.steps, 3)), args.warmup)
         results[qname] = r
         op.close()
+    if args.dump_outputs:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for qname, r in results.items():
+            for name, a in r.pop("outputs").items():
+                np.save(os.path.join(args.dump_outputs, f"{qname}_{name}.npy"), a)
     helm = affine = small = refined = config5 = None
     if not args.no_variants:
         helm = measure_helmholtz(dc, torch, ctx, stream)
