@@ -47,6 +47,13 @@ class PeerInfo(C.Structure):
                 ("rank", C.c_int32), ("device", C.c_int32)]
 
 
+class MgParams(C.Structure):
+    """bp5_mg_params_t: zero selects the default."""
+    _fields_ = [("max_levels", C.c_int32), ("smoothing_degree", C.c_int32), ("smoothing_range", C.c_double),
+                ("eig_iterations", C.c_int32), ("coarse_max_its", C.c_int32), ("coarse_tol", C.c_double),
+                ("reserved", C.c_int32 * 4)]
+
+
 class Bp5Error(RuntimeError):
     def __init__(self, code, msg):
         super().__init__(f"bp5 error {code}: {msg}")
@@ -137,6 +144,20 @@ ABI = [
     ("bp5_vector_compress_add", C.c_int, [_vp, _vp]),
     ("bp5_peer_cg_solve_host", C.c_int, [_vp, _vp, _vp, C.c_int64, C.c_int, C.c_int, C.c_double, C.c_int,
                                          C.POINTER(C.c_int), _dp]),
+    ("bp5_mg_create", C.c_int, [_vp, C.POINTER(MgParams), C.POINTER(_vp)]),
+    ("bp5_mg_destroy", C.c_int, [_vp]),
+    ("bp5_mg_n_levels", C.c_int, [_vp, C.POINTER(C.c_int)]),
+    ("bp5_mg_level_operator", C.c_int, [_vp, C.c_int, C.POINTER(_vp)]),
+    ("bp5_mg_get_lambda_max", C.c_int, [_vp, C.c_int, _dp]),
+    ("bp5_mg_set_lambda_max", C.c_int, [_vp, C.c_int, C.c_double]),
+    ("bp5_mg_prolongate", C.c_int, [_vp, C.c_int, _vp, _vp]),
+    ("bp5_mg_restrict", C.c_int, [_vp, C.c_int, _vp, _vp]),
+    ("bp5_mg_smooth", C.c_int, [_vp, C.c_int, _vp, _vp]),
+    ("bp5_mg_vcycle", C.c_int, [_vp, _vp, _vp]),
+    ("bp5_mg_cg_solve", C.c_int, [_vp, _vp, _vp, C.c_int, C.c_double, C.c_int, C.POINTER(C.c_int), _dp, _dp,
+                                  C.c_int]),
+    ("bp5_mg_profile", C.c_int, [_vp, C.c_int]),
+    ("bp5_mg_profile_result", C.c_int, [_vp, _dp, C.POINTER(C.c_int64)]),
 ]
 
 
@@ -371,6 +392,119 @@ class PoissonOperator:
             self.h = _vp()
 
 
+class _LevelOperator(PoissonOperator):
+    """A multigrid level's operator: owned by the Multigrid object (close() does not destroy it)."""
+
+    def __init__(self, ctx, handle, problem):
+        self.ctx, self.problem, self.h = ctx, problem, handle
+        s = [C.c_int64() for _ in range(4)]
+        _check(lib().bp5_operator_sizes(self.h, *[C.byref(v) for v in s]))
+        self.n_owned, self.n_ghost, self.n_global, self.n_cells = [v.value for v in s]
+        self._zero = True
+
+    def close(self):
+        self.h = _vp()
+
+
+class Multigrid:
+    """Geometric multigrid V-cycle (Chebyshev-Jacobi smoothing, CG on the coarsest level) on the levels of `op`'s
+    mesh: PreconditionMG with MGTransferMatrixFree, PreconditionChebyshev and MGCoarseGridIterativeSolver.
+    One block, conforming mesh, stored geometry, default cell order.  `op` must outlive this object.
+
+    params (0 or None: default): max_levels, smoothing_degree (5), smoothing_range (15), eig_iterations (12),
+    coarse_tol (1e-6, relative), coarse_max_its (1000)."""
+
+    _INT = ("max_levels", "smoothing_degree", "eig_iterations", "coarse_max_its")
+    _FLOAT = ("smoothing_range", "coarse_tol")
+
+    def __init__(self, op, **params):
+        unknown = set(params) - set(self._INT) - set(self._FLOAT)
+        if unknown:
+            raise TypeError(f"unknown multigrid parameter(s): {sorted(unknown)}")
+        prm = MgParams()
+        for k, v in params.items():
+            if v is None:
+                continue
+            if k in self._INT:
+                if int(v) != v or v < 0:
+                    raise ValueError(f"{k} must be a non-negative integer (0: default), got {v!r}")
+                setattr(prm, k, int(v))
+            else:
+                if not np.isfinite(v) or v < 0:
+                    raise ValueError(f"{k} must be a non-negative number (0: default), got {v!r}")
+                setattr(prm, k, float(v))
+        if prm.smoothing_range != 0.0 and prm.smoothing_range <= 1.0:
+            raise ValueError("smoothing_range must exceed 1")
+        if not isinstance(op, PoissonOperator):
+            raise TypeError("Multigrid needs a PoissonOperator")
+        self.op, self.ctx = op, op.ctx
+        self.h = _vp()
+        _check(lib().bp5_mg_create(op.h, C.byref(prm), C.byref(self.h)))
+        n = C.c_int()
+        _check(lib().bp5_mg_n_levels(self.h, C.byref(n)))
+        self.n_levels = n.value
+        self._levels = {}
+
+    def level_operator(self, level):
+        """the operator of `level` (n_levels - 1 is the caller's)"""
+        if level == self.n_levels - 1:
+            return self.op
+        if level not in self._levels:
+            h = _vp()
+            _check(lib().bp5_mg_level_operator(self.h, int(level), C.byref(h)))
+            prob = Problem.from_buffer_copy(self.op.problem)
+            c = self.op.problem.cells
+            f = 2 ** (self.n_levels - 1 - level)
+            for d in range(3):
+                prob.cells[d] = c[d] // f
+            self._levels[level] = _LevelOperator(self.ctx, h, prob)
+        return self._levels[level]
+
+    def lambda_max(self, level):
+        """estimate of the largest eigenvalue of D^-1 A on `level` >= 1 (the smoother uses 1.2 times it)"""
+        out = C.c_double()
+        _check(lib().bp5_mg_get_lambda_max(self.h, int(level), C.byref(out)))
+        return out.value
+
+    def set_lambda_max(self, level, value):
+        _check(lib().bp5_mg_set_lambda_max(self.h, int(level), float(value)))
+
+    def prolongate(self, fine_level, dst, src):
+        """dst (level fine_level) = P src (level fine_level - 1)"""
+        _check(lib().bp5_mg_prolongate(self.h, int(fine_level), dst.h, src.h))
+
+    def restrict(self, fine_level, dst, src):
+        """dst (level fine_level - 1) = P^T src, Dirichlet rows zero"""
+        _check(lib().bp5_mg_restrict(self.h, int(fine_level), dst.h, src.h))
+
+    def smooth(self, level, x, b):
+        """Chebyshev smoothing of A x = b on `level` >= 1 from the x given"""
+        _check(lib().bp5_mg_smooth(self.h, int(level), x.h, b.h))
+
+    def vmult(self, dst, src):
+        """dst = V-cycle(src)"""
+        _check(lib().bp5_mg_vcycle(self.h, dst.h, src.h))
+
+    def profile(self, enable=True):
+        _check(lib().bp5_mg_profile(self.h, int(enable)))
+
+    def profile_result(self):
+        """({level: {"operator", "transfer", "vector", "coarse"} ms}, V-cycles) since the last call"""
+        ms = np.zeros(4 * self.n_levels)
+        n = C.c_int64()
+        _check(lib().bp5_mg_profile_result(self.h, ms.ctypes.data_as(_dp), C.byref(n)))
+        keys = ("operator", "transfer", "vector", "coarse")
+        return {l: dict(zip(keys, ms[4 * l: 4 * l + 4].tolist())) for l in range(self.n_levels)}, n.value
+
+    def close(self):
+        for L in self._levels.values():
+            L.close()
+        self._levels = {}
+        if self.h:
+            lib().bp5_mg_destroy(self.h)
+            self.h = _vp()
+
+
 class SolverControl:
     """SolverControl(max_its, tol): failure at max_its (step-64/step-64.cu:513)."""
     kind = CONTROL_SOLVER
@@ -402,6 +536,19 @@ class _SolverBase:
         c = self.control
         its, val = C.c_int(0), C.c_double(0.0)
         hist = np.full(c.max_its + 2, np.nan) if history else None
+        if isinstance(preconditioner, Multigrid):
+            if self.variant != CG_STANDARD:
+                raise Bp5Error(ERR_UNSUPPORTED, "a multigrid preconditioner needs the standard CG (SolverCG); "
+                                                "the merged variant takes a diagonal only")
+            if A is not preconditioner.op:
+                raise ValueError("the multigrid preconditioner was built on a different operator")
+            rc = lib().bp5_mg_cg_solve(preconditioner.h, x.h, b.h, c.kind, c.tol, c.max_its, C.byref(its),
+                                       C.byref(val), hist.ctypes.data_as(_dp) if hist is not None else None,
+                                       len(hist) if hist is not None else 0)
+            c._last_step, c._last_value = its.value, val.value
+            c.history = hist[: its.value + 1] if hist is not None else None
+            _check(rc)
+            return
         rc = lib().bp5_cg_solve(A.h, x.h, b.h, preconditioner.h if preconditioner is not None else None,
                                 self.variant, c.kind, c.tol, c.max_its, C.byref(its), C.byref(val),
                                 hist.ctypes.data_as(_dp) if hist is not None else None,

@@ -64,6 +64,7 @@ void make_tables(int degree, int quadrature, Tables1D &t);
 void gauss_rule01(int n, double *x, double *w);
 void lobatto_rule01(int n, double *x, double *w);
 void lagrange_eval(int n, const double *nodes, double x, double *val, double *der);
+void parent_child_interp(const Tables1D &t, double (*out)[kMaxN * kMaxN]);   // [s][a*n + b] = l_b((s + xi_a) / 2)
 
 // ---- handles ---------------------------------------------------------------
 }  // namespace bp5

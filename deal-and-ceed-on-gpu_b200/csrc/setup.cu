@@ -806,12 +806,7 @@ int operator_setup_hanging(bp5_operator_t op) {
   op->n_constrained = (int64_t)cons.size();
   BP5_CUDA(cudaMalloc(&op->constrained, sizeof(int) * std::max<size_t>(cons.size(), 1)));
   BP5_CUDA(cudaMemcpyAsync(op->constrained, cons.data(), sizeof(int) * cons.size(), cudaMemcpyHostToDevice, ctx->stream));
-  for (int s = 0; s < 2; ++s)
-    for (int a = 0; a < n; ++a) {
-      double val[kMaxN], der[kMaxN];
-      lagrange_eval(n, op->tab.xi, 0.5 * (s + op->tab.xi[a]), val, der);
-      for (int b = 0; b < n; ++b) op->hanging_interp[s][a * n + b] = val[b];
-    }
+  parent_child_interp(op->tab, op->hanging_interp);
   // ---- the tuned kernel's view of the same cells (apply.cuh, HANG).
   // The numbering is piecewise lexicographic: a cell without a constrained face whose n^3 indices are
   // base + i + j sy + k sz gets the affine descriptor (base >= 0) and the class of its stride pair (at most 8 classes,

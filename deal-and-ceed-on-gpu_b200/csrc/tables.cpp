@@ -95,6 +95,18 @@ void lagrange_eval(int n, const double *nodes, double x, double *val, double *de
   }
 }
 
+// 1D parent-to-child interpolation: out[s][a * n + b] = l_b((s + xi_a) / 2), the value of the parent's basis
+// function b at node a of child s.  Hanging-node constraints and the multigrid transfer both use it.
+void parent_child_interp(const Tables1D &t, double (*out)[kMaxN * kMaxN]) {
+  const int n = t.n;
+  for (int s = 0; s < 2; ++s)
+    for (int a = 0; a < n; ++a) {
+      double val[kMaxN], der[kMaxN];
+      lagrange_eval(n, t.xi, 0.5 * (s + t.xi[a]), val, der);
+      for (int b = 0; b < n; ++b) out[s][a * n + b] = val[b];
+    }
+}
+
 void make_tables(int degree, int quadrature, Tables1D &t) {
   std::memset(&t, 0, sizeof(t));
   const int n = degree + 1;

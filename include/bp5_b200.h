@@ -327,6 +327,63 @@ int bp5_vector_compress_add(bp5_operator_t op, bp5_vector_t vec);
 int bp5_peer_cg_solve_host(bp5_operator_t op, double *x_host, const double *b_host, int64_t n, int x0_is_zero,
                            int control, double tol, int max_its, int *last_step, double *last_value);
 
+/* ---- geometric multigrid: Chebyshev-Jacobi V-cycle as a CG preconditioner ------------------ */
+/* The setup deal.II users pair with a matrix-free operator (MGTransferMatrixFree + PreconditionChebyshev +
+ * MGCoarseGridIterativeSolver inside PreconditionMG) for one block, conforming mesh, stored geometry, default cell
+ * order: every other operator gets BP5_ERR_UNSUPPORTED from bp5_mg_create.
+ *   levels      level n_levels-1 is the caller's operator (not owned; it must outlive the multigrid object); level
+ *               l-1 is the same problem with every cells[d] halved, down to a mesh with an odd or unit cell count
+ *               (or max_levels levels).
+ *   transfer    prolongation P = nodal interpolation coarse -> fine (P_z (x) P_y (x) P_x on the DoF lattice),
+ *               restriction R = P^T followed by zeroed Dirichlet rows; no atomics, bitwise repeatable.
+ *   smoother    Chebyshev iteration of the given degree with D^-1 (inverse diagonal) on levels >= 1, eigenvalue
+ *               range [1.2 lambda / smoothing_range, 1.2 lambda], lambda estimated at set-up by eig_iterations
+ *               Jacobi-preconditioned CG (Lanczos) steps on D^-1 A from a fixed-seed start vector.
+ *   coarse      level 0: standard CG with Jacobi to coarse_tol * |b| or coarse_max_its steps (running out of steps
+ *               is not an error).
+ * Zero in a field of bp5_mg_params_t selects the default; reserved fields must be zero. */
+typedef struct bp5_mg_s *bp5_mg_t;
+typedef struct bp5_mg_params {
+  int32_t max_levels;       /* 0: as many as the mesh allows */
+  int32_t smoothing_degree; /* PreconditionChebyshev::AdditionalData::degree, default 5 */
+  double smoothing_range;   /* ::smoothing_range, default 15 */
+  int32_t eig_iterations;   /* ::eig_cg_n_iterations, default 12 */
+  int32_t coarse_max_its;   /* default 1000 */
+  double coarse_tol;        /* relative, default 1e-6 */
+  int32_t reserved[4];
+} bp5_mg_params_t;
+/* MGLevelObject + MGTransferMatrixFree::build + PreconditionChebyshev::initialize per level [UPSTREAM];
+ * params may be NULL (all defaults) */
+int bp5_mg_create(bp5_operator_t fine_op, const bp5_mg_params_t *params, bp5_mg_t *mg);
+int bp5_mg_destroy(bp5_mg_t mg);
+int bp5_mg_n_levels(bp5_mg_t mg, int *n_levels);
+/* the operator of a level (non-owning; level n_levels-1 is the caller's) */
+int bp5_mg_level_operator(bp5_mg_t mg, int level, bp5_operator_t *op);
+/* PreconditionChebyshev's estimate of the largest eigenvalue of D^-1 A on a level >= 1 (before the factor 1.2);
+ * set replaces it (the smoother then uses the new value) */
+int bp5_mg_get_lambda_max(bp5_mg_t mg, int level, double *lambda);
+int bp5_mg_set_lambda_max(bp5_mg_t mg, int level, double lambda);
+/* MGTransferMatrixFree::prolongate: dst (level fine_level) = P src (level fine_level-1) */
+int bp5_mg_prolongate(bp5_mg_t mg, int fine_level, bp5_vector_t dst, bp5_vector_t src);
+/* MGTransferMatrixFree::restrict_and_add into a zeroed dst: dst (level fine_level-1) = R src, Dirichlet rows 0 */
+int bp5_mg_restrict(bp5_mg_t mg, int fine_level, bp5_vector_t dst, bp5_vector_t src);
+/* PreconditionChebyshev::step on a level >= 1: x <- Chebyshev smoothing of A x = b from the x given (an all-zero x
+ * takes the path without the initial operator application) */
+int bp5_mg_smooth(bp5_mg_t mg, int level, bp5_vector_t x, bp5_vector_t b);
+/* PreconditionMG::vmult: dst = V(src), one V-cycle from a zero initial guess on the finest level */
+int bp5_mg_vcycle(bp5_mg_t mg, bp5_vector_t dst, bp5_vector_t src);
+/* dealii::SolverCG::solve(A, x, b, PreconditionMG) on the finest level; arguments, status codes and history as
+ * bp5_cg_solve (x on entry is the initial guess).  Scalars live on the host: one V-cycle per iteration. */
+int bp5_mg_cg_solve(bp5_mg_t mg, bp5_vector_t x, bp5_vector_t b, int control, double tol, int max_its, int *last_step,
+                    double *last_value, double *history, int history_len);
+/* timing of the V-cycle's parts by CUDA events on the context's stream (off by default).  profile_result
+ * synchronises, writes ms[4 * level + k] for k = 0 operator applications, 1 transfers between the level and the next
+ * coarser one (restriction, zeroed Dirichlet rows, prolongation), 2 Chebyshev and residual vector kernels, 3 coarse
+ * solve (level 0 only),
+ * returns the number of V-cycles since the last call and resets the counters. */
+int bp5_mg_profile(bp5_mg_t mg, int enable);
+int bp5_mg_profile_result(bp5_mg_t mg, double *ms, int64_t *n_vcycles);
+
 #ifdef __cplusplus
 }
 #endif

@@ -463,6 +463,48 @@ template <int dim, int fe_degree, int operator_kind> class MatrixFreeOperator {
  public:
   bool do_zero_out;                                               // bp5/step-64.cu:223
 };
+
+// PreconditionMG<dim, VectorType, MGTransferMatrixFree> with PreconditionChebyshev smoothers (Jacobi inside) and an
+// MGCoarseGridIterativeSolver (CG) [UPSTREAM], all on the library's levels of the operator's mesh: one block,
+// conforming mesh, stored geometry, default cell order.  The operator must outlive the preconditioner.
+template <int dim, int fe_degree, int operator_kind> class MultigridPreconditioner {
+ public:
+  using VectorType = LinearAlgebra::distributed::Vector<double, MemorySpace::CUDA>;
+  struct AdditionalData {                 // field names of PreconditionChebyshev::AdditionalData where they exist
+    unsigned int degree = 5;
+    double smoothing_range = 15.;
+    unsigned int eig_cg_n_iterations = 12;
+    unsigned int max_levels = 0;          // 0: coarsen while every cell count is even
+    double coarse_tolerance = 1e-6;       // relative, MGCoarseGridIterativeSolver's SolverControl
+    unsigned int coarse_max_iterations = 1000;
+  };
+  explicit MultigridPreconditioner(const MatrixFreeOperator<dim, fe_degree, operator_kind> &op,
+                                   const AdditionalData &data = AdditionalData()) : op(op.handle()) {
+    if (op.partitioned()) throw ExcMessage("MultigridPreconditioner: one block only (no multigrid across ranks)");
+    bp5_mg_params_t prm{};
+    prm.max_levels = (int32_t)data.max_levels;
+    prm.smoothing_degree = (int32_t)data.degree;
+    prm.smoothing_range = data.smoothing_range;
+    prm.eig_iterations = (int32_t)data.eig_cg_n_iterations;
+    prm.coarse_max_its = (int32_t)data.coarse_max_iterations;
+    prm.coarse_tol = data.coarse_tolerance;
+    check(bp5_mg_create(this->op, &prm, &h));
+  }
+  MultigridPreconditioner(const MultigridPreconditioner &) = delete;
+  ~MultigridPreconditioner() { bp5_mg_destroy(h); }
+  // PreconditionMG::vmult: dst = one V-cycle applied to src
+  void vmult(VectorType &dst, const VectorType &src) const {
+    check(bp5_mg_vcycle(h, dst.handle(), src.handle()));
+    dst.mark_modified();
+  }
+  unsigned int n_levels() const { int n = 0; check(bp5_mg_n_levels(h, &n)); return (unsigned)n; }
+  bp5_mg_t handle() const { return h; }
+  bp5_operator_t operator_handle() const { return op; }
+
+ private:
+  bp5_operator_t op = nullptr;
+  bp5_mg_t h = nullptr;
+};
 }  // namespace b200
 
 // ------------------------------------------------------------------ solvers
@@ -474,6 +516,14 @@ struct has_native_handle<M, std::void_t<decltype(std::declval<const M &>().handl
                                         decltype(std::declval<const M &>().partitioned())>>
     : std::is_same<decltype(std::declval<const M &>().handle()), bp5_operator_t> {};
 
+// a preconditioner with get_vector() is a DiagonalMatrix; any other one is applied through vmult(dst, src)
+template <typename P, typename = void> struct has_get_vector : std::false_type {};
+template <typename P>
+struct has_get_vector<P, std::void_t<decltype(std::declval<const P &>().get_vector())>> : std::true_type {};
+template <typename P> struct is_multigrid : std::false_type {};
+template <int dim, int fe_degree, int kind>
+struct is_multigrid<MultigridPreconditioner<dim, fe_degree, kind>> : std::true_type {};
+
 template <typename VectorType, int variant> class SolverCGBase {
  public:
   explicit SolverCGBase(SolverControl &cn) : control(cn) {}
@@ -481,6 +531,31 @@ template <typename VectorType, int variant> class SolverCGBase {
 
   template <typename MatrixType, typename PreconditionerType>
   void solve(const MatrixType &A, VectorType &x, const VectorType &b, const PreconditionerType &preconditioner) {
+    if constexpr (has_get_vector<PreconditionerType>::value) {
+      solve_diagonal(A, x, b, preconditioner);
+    } else {
+      static_assert(variant == BP5_CG_STANDARD,
+                    "SolverCGFullMerge takes a DiagonalMatrix preconditioner only: use SolverCG with a multigrid or "
+                    "other vmult preconditioner");
+      if constexpr (has_native_handle<MatrixType>::value && is_multigrid<PreconditionerType>::value) {
+        if (preconditioner.operator_handle() != A.handle())
+          throw ExcMessage("SolverCG: the multigrid preconditioner was built on a different operator");
+        // library operator + library multigrid: the whole loop is one native call
+        int its = 0;
+        double val = 0.0;
+        const int rc = bp5_mg_cg_solve(preconditioner.handle(), x.handle(), b.handle(), control.abi_kind(),
+                                       control.tolerance(), (int)control.max_steps(), &its, &val, nullptr, 0);
+        if (rc == BP5_ERR_DIVIDE_BY_ZERO) { control.record((unsigned)its, val); throw ExcDivideByZero(); }
+        finish(rc, its, val, x);
+      } else {
+        solve_standard_preconditioned(A, x, b, preconditioner);
+      }
+    }
+  }
+
+ protected:
+  template <typename MatrixType, typename PreconditionerType>
+  void solve_diagonal(const MatrixType &A, VectorType &x, const VectorType &b, const PreconditionerType &preconditioner) {
     // the reference passes a DiagonalMatrix of ones (bp5/step-64.cu:428-432) and reads it in every
     // pass; an all-ones diagonal is recognised and not read at all (SURVEY.md 8a, S4)
     const VectorType &diag = preconditioner.get_vector();
@@ -593,6 +668,43 @@ template <typename VectorType, int variant> class SolverCGBase {
       conv = host_check(it, res);
       if (conv != 0) break;
       if (has_diag) { h.equ(1., g); h.scale(diag); } else h.equ(1., g);
+      const double gh_new = g * h;
+      const double beta = gh_new / gh;
+      gh = gh_new;
+      d.sadd(beta, -1., h);
+    }
+    finish(conv == 2 ? BP5_ERR_NO_CONVERGENCE : BP5_OK, (int)it, res, x);
+  }
+
+  // dealii::SolverCG [UPSTREAM] around any operator and any preconditioner with vmult(dst, src)
+  template <typename MatrixType, typename PreconditionerType>
+  void solve_standard_preconditioned(const MatrixType &A, VectorType &x, const VectorType &b,
+                                     const PreconditionerType &preconditioner) {
+    VectorType g, d, h;
+    g.reinit(x); d.reinit(x); h.reinit(x);
+    if (!x.all_zero()) { A.vmult(g, x); g.add(-1., b); } else g.equ(-1., b);
+    double res = g.l2_norm();
+    unsigned it = 0;
+    int conv = host_check(0, res);
+    double gh = 0.;
+    if (conv == 0) {
+      preconditioner.vmult(h, g);
+      d.equ(-1., h);
+      gh = g * h;
+    }
+    while (conv == 0) {
+      ++it;
+      h = 0.;
+      A.vmult(h, d);
+      const double dAd = d * h;
+      if (dAd == 0.) { control.record(it, res); throw ExcDivideByZero(); }
+      const double alpha = gh / dAd;
+      x.add(alpha, d);
+      g.add(alpha, h);
+      res = g.l2_norm();
+      conv = host_check(it, res);
+      if (conv != 0) break;
+      preconditioner.vmult(h, g);
       const double gh_new = g * h;
       const double beta = gh_new / gh;
       gh = gh_new;
