@@ -92,7 +92,6 @@ ABI = [
     ("bp5_operator_l2_norm_sqr", C.c_int, [_vp, _vp, _dp]),
     ("bp5_operator_compute_diagonal", C.c_int, [_vp, _vp, C.c_int]),
     ("bp5_operator_algorithmic_bytes", C.c_int, [_vp, _dp, _dp]),
-    ("bp5_operator_set_option", C.c_int, [_vp, C.c_char_p, C.c_int]),
     ("bp5_operator_profile", C.c_int, [_vp, C.c_int]),
     ("bp5_operator_profile_result", C.c_int, [_vp, C.POINTER(C.c_int64), _dp]),
     ("bp5_operator_kernel_name", C.c_char_p, [_vp]),
@@ -370,9 +369,6 @@ class PoissonOperator:
         a, b = C.c_double(), C.c_double()
         _check(lib().bp5_operator_algorithmic_bytes(self.h, C.byref(a), C.byref(b)))
         return a.value, b.value
-
-    def set_option(self, name, value):
-        _check(lib().bp5_operator_set_option(self.h, name.encode(), int(value)))
 
     def profile(self, enable=True):
         _check(lib().bp5_operator_profile(self.h, int(enable)))

@@ -1,5 +1,4 @@
 // extern "C" entry points declared in include/bp5_b200.h.
-#include <cstdlib>
 #include <cstring>
 #include <new>
 
@@ -29,6 +28,31 @@ using namespace bp5;
     set_error("unexpected C++ exception at the ABI boundary"); \
     return BP5_ERR_INVALID;                                   \
   }
+
+// Host-buffer solves: b and the owned range of x (or zeros when x0_is_zero) go to the operator's staging vectors, whose
+// ghost entries are zero; `solve(x, b)` runs on them, and x comes back unless the solve failed outright.
+template <typename Solve>
+static int solve_host(bp5_operator_t op, double *x_host, const double *b_host, int x0_is_zero, Solve solve) {
+  bp5_context_t ctx = op->ctx;
+  const int64_t n = op->n_owned;
+  int rc;
+  if (!op->xh) {
+    if ((rc = bp5_vector_create(ctx, op->n_owned, op->n_ghost, &op->xh))) return rc;
+    if ((rc = bp5_vector_create(ctx, op->n_owned, op->n_ghost, &op->bh))) return rc;
+  }
+  BP5_CUDA(cudaMemcpyAsync(op->bh->d, b_host, sizeof(double) * n, cudaMemcpyHostToDevice, ctx->stream));
+  if (x0_is_zero) {
+    BP5_CUDA(cudaMemsetAsync(op->xh->d, 0, sizeof(double) * (n + op->n_ghost), ctx->stream));
+  } else {
+    BP5_CUDA(cudaMemcpyAsync(op->xh->d, x_host, sizeof(double) * n, cudaMemcpyHostToDevice, ctx->stream));
+    if (op->n_ghost) BP5_CUDA(cudaMemsetAsync(op->xh->d + n, 0, sizeof(double) * op->n_ghost, ctx->stream));
+  }
+  rc = solve(op->xh, op->bh);
+  if (rc != BP5_OK && rc != BP5_ERR_NO_CONVERGENCE) return rc;
+  BP5_CUDA(cudaMemcpyAsync(x_host, op->xh->d, sizeof(double) * n, cudaMemcpyDeviceToHost, ctx->stream));
+  BP5_CUDA(cudaStreamSynchronize(ctx->stream));
+  return rc;
+}
 
 extern "C" {
 
@@ -162,7 +186,6 @@ int bp5_operator_create(bp5_context_t ctx, const bp5_problem_t *pr, bp5_operator
               (long long)(owned + goff));
     return BP5_ERR_UNSUPPORTED;
   }
-  if (const char *sv = getenv("BP5_SLAB")) op->slab_enabled = atoi(sv) != 0;
   int rc;
   if (refined) {
     // hanging nodes: numbering and the generic functor path's arrays only (the tuned kernel handles conforming meshes)
@@ -197,8 +220,6 @@ int bp5_operator_destroy(bp5_operator_t op) {
   cudaFree(op->coords);
   cudaFree(op->constrained);
   cudaFree(op->cg_scalars);
-  if (op->graph_exec) cudaGraphExecDestroy(static_cast<cudaGraphExec_t>(op->graph_exec));
-  slab_destroy(op);
   for (cudaEvent_t e : op->prof_events) cudaEventDestroy(e);
   bp5_vector_destroy(op->g);
   bp5_vector_destroy(op->d);
@@ -369,13 +390,6 @@ int bp5_operator_algorithmic_bytes(bp5_operator_t op, double *per_vmult, double 
   if (per_vmult) *per_vmult = 16.0 * (double)op->n_owned + metric;
   if (per_cg_it) *per_cg_it = 72.0 * (double)op->n_owned + metric;
   return BP5_OK;
-}
-
-int bp5_operator_set_option(bp5_operator_t op, const char *name, int value) {
-  BP5_REQUIRE(op && name, "null argument");
-  if (std::strcmp(name, "slab_pipeline") == 0) { op->slab_enabled = value != 0; return BP5_OK; }
-  set_error("unknown option '%s'", name);
-  return BP5_ERR_INVALID;
 }
 
 int bp5_operator_profile(bp5_operator_t op, int enable) {
@@ -552,20 +566,9 @@ int bp5_cg_solve_host(bp5_operator_t op, double *x_host, const double *b_host, i
   BP5_REQUIRE(op && x_host && b_host, "null argument");
   BP5_REQUIRE(n == op->n_owned && op->n_ghost == 0, "host solve needs a single block and n == n_dofs");
   BP5_CUDA(cudaSetDevice(op->ctx->device));
-  bp5_context_t ctx = op->ctx;
-  if (!op->xh) {
-    int rc;
-    if ((rc = bp5_vector_create(ctx, n, 0, &op->xh))) return rc;
-    if ((rc = bp5_vector_create(ctx, n, 0, &op->bh))) return rc;
-  }
-  BP5_CUDA(cudaMemcpyAsync(op->bh->d, b_host, sizeof(double) * n, cudaMemcpyHostToDevice, ctx->stream));
-  if (x0_is_zero) BP5_CUDA(cudaMemsetAsync(op->xh->d, 0, sizeof(double) * n, ctx->stream));
-  else BP5_CUDA(cudaMemcpyAsync(op->xh->d, x_host, sizeof(double) * n, cudaMemcpyHostToDevice, ctx->stream));
-  const int rc = cg_solve(op, op->xh, op->bh, nullptr, variant, control, tol, max_its, last_step, last_value, nullptr, 0);
-  if (rc != BP5_OK && rc != BP5_ERR_NO_CONVERGENCE) return rc;
-  BP5_CUDA(cudaMemcpyAsync(x_host, op->xh->d, sizeof(double) * n, cudaMemcpyDeviceToHost, ctx->stream));
-  BP5_CUDA(cudaStreamSynchronize(ctx->stream));
-  return rc;
+  return solve_host(op, x_host, b_host, x0_is_zero, [&](bp5_vector_t x, bp5_vector_t b) {
+    return cg_solve(op, x, b, nullptr, variant, control, tol, max_its, last_step, last_value, nullptr, 0);
+  });
   BP5_ABI_GUARD_END
 }
 
@@ -808,20 +811,9 @@ int bp5_peer_cg_solve_host(bp5_operator_t op, double *x_host, const double *b_ho
   BP5_REQUIRE(op && x_host && b_host, "null argument");
   BP5_REQUIRE(n == op->n_owned, "host buffers hold this block's owned range: n == n_owned");
   BP5_CUDA(cudaSetDevice(op->ctx->device));
-  bp5_context_t ctx = op->ctx;
-  int rc;
-  if (!op->xh) {
-    if ((rc = bp5_vector_create(ctx, op->n_owned, op->n_ghost, &op->xh))) return rc;
-    if ((rc = bp5_vector_create(ctx, op->n_owned, op->n_ghost, &op->bh))) return rc;
-  }
-  BP5_CUDA(cudaMemcpyAsync(op->bh->d, b_host, sizeof(double) * n, cudaMemcpyHostToDevice, ctx->stream));
-  BP5_CUDA(cudaMemsetAsync(op->xh->d, 0, sizeof(double) * (op->n_owned + op->n_ghost), ctx->stream));
-  if (!x0_is_zero) BP5_CUDA(cudaMemcpyAsync(op->xh->d, x_host, sizeof(double) * n, cudaMemcpyHostToDevice, ctx->stream));
-  rc = cg_solve_peer(op, op->xh, op->bh, nullptr, control, tol, max_its, last_step, last_value, nullptr, 0);
-  if (rc != BP5_OK && rc != BP5_ERR_NO_CONVERGENCE) return rc;
-  BP5_CUDA(cudaMemcpyAsync(x_host, op->xh->d, sizeof(double) * n, cudaMemcpyDeviceToHost, ctx->stream));
-  BP5_CUDA(cudaStreamSynchronize(ctx->stream));
-  return rc;
+  return solve_host(op, x_host, b_host, x0_is_zero, [&](bp5_vector_t x, bp5_vector_t b) {
+    return cg_solve_peer(op, x, b, nullptr, control, tol, max_its, last_step, last_value, nullptr, 0);
+  });
   BP5_ABI_GUARD_END
 }
 

@@ -127,7 +127,7 @@ int apply_cell_loop(bp5_operator_t op, double *dst, const double *src, bool over
                     int which) {
   BP5_REQUIRE(dot_partials == nullptr || overwrite_interior, "the fused dot product needs the overwrite kernel");
   const int mode = dot_partials ? 2 : (overwrite_interior ? 1 : 0);
-  if (op->hanging && !op->range_query) {
+  if (op->hanging) {
     // locally refined mesh: the tiles with constrained / table cells through the kernel with the constraint exchange,
     // then all others; the per-CTA partial sums of the fused dot product one group after the other
     BP5_REQUIRE(op->range_begin < 0 && which == 0, "locally refined meshes run whole cell loops only");
@@ -137,7 +137,7 @@ int apply_cell_loop(bp5_operator_t op, double *dst, const double *src, bool over
     op->apply_grid += first;
     return rc;
   }
-  if (op->prob.cell_order != BP5_CELL_ORDER_COLORED || op->range_query) return apply_dispatch(op, dst, src, mode, dot_partials, which);
+  if (op->prob.cell_order != BP5_CELL_ORDER_COLORED) return apply_dispatch(op, dst, src, mode, dot_partials, which);
   // coloured cell order: one launch per colour over that colour's tiles, in a fixed order on one stream; the
   // per-CTA partial sums of the fused dot product are laid out colour after colour.
   BP5_REQUIRE(op->range_begin < 0 && which == 0, "the coloured cell order runs whole cell loops only");

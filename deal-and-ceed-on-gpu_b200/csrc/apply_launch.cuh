@@ -43,9 +43,8 @@ static int launch(bp5_operator_t op, double *dst, const double *src, double *dot
   prm.src = src; prm.dst = dst;
   prm.tile_begin = which == 2 ? op->n_boundary_tiles : 0;
   prm.n_tiles = which == 1 ? op->n_boundary_tiles : op->n_tiles;      // end of the range
-  if (op->range_begin >= 0) { prm.tile_begin = op->range_begin; prm.n_tiles = op->range_end; }   // slab pipeline
-  if (op->range_query) { op->apply_grid_full = blocks_per_sm * op->ctx->sm_count; return BP5_OK; }
-  cudaStream_t stream = op->launch_stream ? op->launch_stream : op->ctx->stream;
+  if (op->range_begin >= 0) { prm.tile_begin = op->range_begin; prm.n_tiles = op->range_end; }   // explicit tile range
+  cudaStream_t stream = op->ctx->stream;
   prm.sy = op->od[0]; prm.sz = op->od[0] * op->od[1];
   if (prm.n_tiles <= prm.tile_begin) { op->apply_grid = 0; return BP5_OK; }
   prm.skip = op->skip_flag;

@@ -16,7 +16,7 @@ struct CgState {
 };
 
 // SolverControl::check / IterationNumberControl::check [UPSTREAM]
-__device__ __forceinline__ int control_check(int control, int step, int max_its, double value, double tol) {
+__host__ __device__ __forceinline__ int control_check(int control, int step, int max_its, double value, double tol) {
   if (control == BP5_CONTROL_ITERATION_NUMBER && step >= max_its) return 1;
   if (value <= tol) return 1;
   if (step >= max_its || isnan(value)) return 2;

@@ -66,6 +66,17 @@ void lobatto_rule01(int n, double *x, double *w);
 void lagrange_eval(int n, const double *nodes, double x, double *val, double *der);
 void parent_child_interp(const Tables1D &t, double (*out)[kMaxN * kMaxN]);   // [s][a*n + b] = l_b((s + xi_a) / 2)
 
+// device scratch of one CG solve (cg.cu): [CgState | dots partials | cell-kernel p.v partials | Dirichlet correction
+// partials | update-kernel r.r partials | residual history]
+struct CgState;
+struct CgBuffers {
+  CgState *st;
+  double *partials;    // [kCgBlocks][7]
+  double *ph;          // [kApplyPartialCap + kConstrainedPartials]
+  double *rr;          // [kUpdatePartialCap][2]
+  double *hist;        // [hist_len] or nullptr
+};
+
 // ---- handles ---------------------------------------------------------------
 }  // namespace bp5
 
@@ -147,6 +158,7 @@ struct bp5_operator_s {
   size_t cg_scalars_bytes = 0;
   bp5_vector_t cg_x = nullptr, cg_diag = nullptr;   // stepwise CG: caller's solution / diagonal
   int cg_hist_len = 0;
+  bp5::CgBuffers cg_buf{};      // stepwise CG: cg_scalars as laid out by cg_step_begin
   bool cg_ph_valid = false;     // stepwise CG: the cell kernel left d.h partials for the next dots step
   int cg_update_grid = 0;       // stepwise CG: blocks (= r.r partials) of the last update step
   // live per-launch timing of the cell kernel (bench.py roofline): events around every launch
@@ -156,17 +168,9 @@ struct bp5_operator_s {
   void *peer = nullptr;          // peer-memory transport state (peer.cu), or null
   bool peer_connected = false;
   const int *skip_flag = nullptr; // device word: when non-zero the cell loop is a no-op (CG converged)
-  // slab-pipelined CG iteration (slab.cu): overrides of the next cell-kernel launch, plan, cached graph
+  // overrides of the next cell-kernel launch (peer-memory CG, coloured cell order)
   long long range_begin = -1, range_end = -1;   // tile range instead of `which`
   int grid_cap = 0;                             // upper bound of the cell kernel's grid (colour passes), 0 = none
-  bool range_query = false;                     // only size the persistent grid (apply_grid_full), no launch
-  cudaStream_t launch_stream = nullptr;         // instead of the context's stream
-  int apply_grid_full = 0;                      // CTAs of a full launch of the CG-mode cell kernel
-  bool slab_enabled = false;                    // bp5_operator_set_option("slab_pipeline", 1) or BP5_SLAB=1
-  void *slab = nullptr;                         // SlabPlan
-  void *graph_exec = nullptr;                   // cudaGraphExec_t of the last slab-pipelined batch
-  int64_t graph_launches = 0;
-  const void *graph_key[4] = {nullptr, nullptr, nullptr, nullptr}, *graph_key_cached[4] = {nullptr, nullptr, nullptr, nullptr};
 };
 
 namespace bp5 {
@@ -194,11 +198,6 @@ int apply_cell_loop_otfg(bp5_operator_t op, double *dst, const double *src, int 
 int apply_copy_constrained_dot(bp5_operator_t op, double *dst, const double *src, double *partials);
 int apply_zero_skeleton(bp5_operator_t op, double *dst);
 int apply_copy_constrained(bp5_operator_t op, double *dst, const double *src);
-// slab.cu
-bool slab_supported(bp5_operator_t op);
-void slab_destroy(bp5_operator_t op);
-int slab_enqueue_iteration(bp5_operator_t op, int cur, void *state, double *hist_dev, double *g, double *d, double *h,
-                           double *x, const double *diag);
 // vector.cu
 int vec_fill(bp5_context_t ctx, double *d, int64_t n, double v);
 int vec_axpy(bp5_context_t ctx, double *y, double s, double a, const double *x, int64_t n, int mode);
@@ -228,6 +227,12 @@ int peer_check(bp5_operator_t op);
 int cg_solve_peer(bp5_operator_t op, bp5_vector_t x, bp5_vector_t b, bp5_vector_t diag, int control, double tol,
                   int max_its, int *last_step, double *last_value, double *history, int history_len);
 // cg.cu
+// creates the work vectors g, d, h on first use and grows the device scratch to hold a residual history of hist_len;
+// cb (may be null) receives its layout
+int cg_buffers(bp5_operator_t op, int hist_len, CgBuffers *cb);
+// return code and error text of a CG that ended in CgState::state `state` (1 success, 2 no convergence, 3 d.Ad == 0)
+// after `it` iterations at residual `res`
+int cg_status(int state, int it, double res);
 int cg_step_begin(bp5_operator_t op, bp5_vector_t x, bp5_vector_t b, bp5_vector_t diag, int control, double tol,
                   int max_its, double res0, int history_len);
 int cg_step_update(bp5_operator_t op, int iteration);

@@ -18,6 +18,7 @@
 #include <vector>
 
 #include "apply.cuh"
+#include "cg_state.cuh"
 #include "common.h"
 
 namespace bp5 {
@@ -673,17 +674,11 @@ int bp5_mg_cg_solve(bp5_mg_t mg, bp5_vector_t x, bp5_vector_t b, int control, do
   } else if ((rc = vec_axpy(ctx, g, 0.0, -1.0, b->d, n, 1))) {
     return rc;
   }
-  auto check = [&](int step, double value) {
-    if (control == BP5_CONTROL_ITERATION_NUMBER && step >= max_its) return 1;
-    if (value <= tol) return 1;
-    if (step >= max_its || std::isnan(value)) return 2;
-    return 0;
-  };
   double gg = 0.0;
   if ((rc = vec_dot(ctx, g, g, n, &gg))) return rc;
   double res = std::sqrt(gg);
   if (history && history_len > 0) history[0] = res;
-  int it = 0, conv = check(0, res);
+  int it = 0, conv = control_check(control, 0, max_its, res, tol);
   double gh = 0.0;
   if (conv == 0) {
     if ((rc = vcycle(mg, top, mg->h, mg->g))) return rc;       // h = M^-1 g
@@ -699,8 +694,7 @@ int bp5_mg_cg_solve(bp5_mg_t mg, bp5_vector_t x, bp5_vector_t b, int control, do
     if (dad == 0.0) {
       if (last_step) *last_step = it;
       if (last_value) *last_value = res;
-      set_error("ExcDivideByZero: d.Ad == 0 at iteration %d", it);
-      return BP5_ERR_DIVIDE_BY_ZERO;
+      return cg_status(3, it, res);
     }
     const double alpha = gh / dad;
     if ((rc = vec_axpy(ctx, x->d, 0.0, alpha, d, n, 0))) return rc;
@@ -708,7 +702,7 @@ int bp5_mg_cg_solve(bp5_mg_t mg, bp5_vector_t x, bp5_vector_t b, int control, do
     if ((rc = vec_dot(ctx, g, g, n, &gg))) return rc;
     res = std::sqrt(gg);
     if (history && it < history_len) history[it] = res;
-    if ((conv = check(it, res)) != 0) break;
+    if ((conv = control_check(control, it, max_its, res, tol)) != 0) break;
     if ((rc = vcycle(mg, top, mg->h, mg->g))) return rc;
     if (mg->profile) mg->n_vcycles++;
     const double gh_old = gh;
@@ -718,11 +712,7 @@ int bp5_mg_cg_solve(bp5_mg_t mg, bp5_vector_t x, bp5_vector_t b, int control, do
   BP5_CUDA(cudaStreamSynchronize(ctx->stream));
   if (last_step) *last_step = it;
   if (last_value) *last_value = res;
-  if (conv == 2) {
-    set_error("NoConvergence: step %d, residual %.17g", it, res);
-    return BP5_ERR_NO_CONVERGENCE;
-  }
-  return BP5_OK;
+  return cg_status(conv, it, res);
   BP5_MG_GUARD_END
 }
 

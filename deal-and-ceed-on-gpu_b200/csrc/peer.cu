@@ -271,11 +271,7 @@ int peer_export(bp5_operator_t op, int rank, int world, bp5_peer_info_t *out) {
   BP5_REQUIRE(world >= 1 && world <= kPeerMaxWorld && rank >= 0 && rank < world, "bad rank / world size");
   bp5_context_t ctx = op->ctx;
   int rc;
-  if (!op->d) {   // the CG work vectors double as the exchange vectors
-    if ((rc = bp5_vector_create(ctx, op->n_owned, op->n_ghost, &op->g))) return rc;
-    if ((rc = bp5_vector_create(ctx, op->n_owned, op->n_ghost, &op->d))) return rc;
-    if ((rc = bp5_vector_create(ctx, op->n_owned, op->n_ghost, &op->h))) return rc;
-  }
+  if ((rc = cg_buffers(op, 0, nullptr))) return rc;   // the CG work vectors double as the exchange vectors
   if (!op->peer) {
     PeerState *ps = new PeerState;
     int64_t sc[8], so[8], rcv[8], ro[8];

@@ -136,12 +136,6 @@ int bp5_operator_l2_norm_sqr(bp5_operator_t op, bp5_vector_t u, double *out);
 int bp5_operator_compute_diagonal(bp5_operator_t op, bp5_vector_t diag, int invert);
 /* algorithmic bytes of one vmult over this block (SURVEY 8d: 16 + 48 r per DoF) */
 int bp5_operator_algorithmic_bytes(bp5_operator_t op, double *bytes_per_vmult, double *bytes_per_cg_it);
-/* tuning switches.  "slab_pipeline" (default 0): 1 makes bp5_cg_solve(BP5_CG_MERGED) on a single block run every
- * iteration as a pipeline of slabs -- vector update, cell loop and dot products a few slabs of cells apart, each an
- * ordinary kernel on its own stream -- so that the vectors change hands in L2 (7 instead of 12 vector passes
- * through HBM per iteration).  Same results; measured slower than the separate full-length kernels on B200
- * (DESIGN.md section 3.4), hence opt-in. */
-int bp5_operator_set_option(bp5_operator_t op, const char *name, int value);
 /* live timing of the cell kernel: when enabled, every launch of the hot kernel
  * is bracketed by CUDA events on the context's stream; profile_result
  * synchronises, returns the number of launches and their summed device time
