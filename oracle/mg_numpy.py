@@ -144,29 +144,39 @@ class NumpyMG:
         return pcg(lambda v: self.A[-1] @ v, self.vcycle, b, tol, max_its)
 
 
-def pcg(apply_A, apply_M, b, tol, max_its):
-    """dealii::SolverCG with a preconditioner from x = 0 (stops at |g| <= tol or max_its)"""
-    x = np.zeros_like(b)
-    g = -b.copy()
-    res = np.linalg.norm(g)
+def dot(a, b):
+    """a . b through numpy's own loops: a BLAS level-1 call leaves OpenBLAS's worker threads spinning, and they slow
+    the next OpenMP oracle vmult (mg_matfree.py) by an order of magnitude"""
+    return float(np.einsum("i,i->", a, b))
+
+
+def pcg(apply_A, apply_M, b, tol, max_its, x0=None):
+    """dealii::SolverCG with a preconditioner from x0 (None: zero; stops at |g| <= tol or max_its)"""
+    if x0 is None:
+        x = np.zeros_like(b)
+        g = -b.copy()
+    else:
+        x = np.array(x0, dtype=np.float64)
+        g = apply_A(x) - b
+    res = np.sqrt(dot(g, g))
     hist = [res]
     if res <= tol or max_its == 0:
         return x, 0, hist
     h = apply_M(g)
     d = -h
-    gh = g @ h
+    gh = dot(g, h)
     it = 0
     while True:
         it += 1
         ad = apply_A(d)
-        alpha = gh / (d @ ad)
+        alpha = gh / dot(d, ad)
         x += alpha * d
         g += alpha * ad
-        res = np.linalg.norm(g)
+        res = np.sqrt(dot(g, g))
         hist.append(res)
         if res <= tol or it >= max_its:
             break
         h = apply_M(g)
-        gh_old, gh = gh, g @ h
+        gh_old, gh = gh, dot(g, h)
         d = (gh / gh_old) * d - h
     return x, it, hist
