@@ -383,10 +383,9 @@ int bp5_operator_algorithmic_bytes(bp5_operator_t op, double *per_vmult, double 
   // CG: read {x,r,p,h,diag} + write {x,r,p,h} = 72, plus the metric.
   const double n3 = (double)op->n * op->n * op->n;
   // stored metric: 8 bytes per plane per quadrature point; on the fly: three coordinates per local DoF
-  const double metric = op->metric_path == 3 ? 0.0        // affine mesh, geometry on the fly: three constants
-                        : op->prob.geometry_mode == BP5_GEOM_ON_THE_FLY
-                            ? 24.0 * (double)(op->n_owned + op->n_ghost)
-                            : 8.0 * op->metric_planes * n3 * (double)op->n_cells;
+  const double metric = op->cell_kernel == CellKernel::kAffine ? 0.0      // geometry on the fly: three constants
+                        : op->cell_kernel == CellKernel::kStored ? 8.0 * op->metric_planes * n3 * (double)op->n_cells
+                                                                 : 24.0 * (double)(op->n_owned + op->n_ghost);
   if (per_vmult) *per_vmult = 16.0 * (double)op->n_owned + metric;
   if (per_cg_it) *per_cg_it = 72.0 * (double)op->n_owned + metric;
   return BP5_OK;

@@ -5,121 +5,72 @@
 
 namespace bp5 {
 
-static int cells_per_tile_for(int p) {
-  switch (p) {
-    case 1: return TileCells<1>::value; case 2: return TileCells<2>::value;
-    case 3: return TileCells<3>::value; case 4: return TileCells<4>::value;
-    case 5: return TileCells<5>::value; case 6: return TileCells<6>::value;
-    case 7: return TileCells<7>::value; case 8: return TileCells<8>::value;
-  }
-  return 0;
-}
-
 int apply_choose(bp5_operator_t op) {
-  int cpt = cells_per_tile_for(op->p);
-  BP5_REQUIRE(cpt > 0, "degree must be 1..8");
-  if (op->prob.geometry_mode == BP5_GEOM_ON_THE_FLY) {
+  const bool gll = op->prob.quadrature == BP5_QUAD_GLL, helm = op->prob.operator_kind == BP5_OP_HELMHOLTZ;
+  if (op->prob.geometry_mode != BP5_GEOM_ON_THE_FLY)
+    op->cell_kernel = CellKernel::kStored;
+  else if (op->prob.deformation == 0 && !helm)   // undeformed (axis-parallel) mesh: no coordinate gathers
+    op->cell_kernel = CellKernel::kAffine;
+  else if (gll && !helm && op->p <= 4)
     // collocation + Poisson: the four-fields-at-once kernel (apply_otf.cuh) up to p = 4, the general kernel above
     // (p = 5: 21.9 against 19.9, p = 6: 23.3 against 20.9 GDoF/s per vmult on a deformed mesh)
-    op->otf_general = !(op->prob.quadrature == BP5_QUAD_GLL && op->prob.operator_kind == BP5_OP_POISSON) || op->p >= 5;
-#ifdef BP5_TUNING_ENV        // tuning builds only
-    if (const char *v = getenv("BP5_OTF_GENERAL"))   // 0 / 1: which kernel takes collocation + Poisson
-      op->otf_general = atoi(v) != 0 || !(op->prob.quadrature == BP5_QUAD_GLL && op->prob.operator_kind == BP5_OP_POISSON);
-#endif
-    switch (op->p) {
-#define BP5_OTF_CASE(P) case P: cpt = op->otf_general ? OtfgTileCells<P>::value : OtfTileCells<P>::value; break;
-      BP5_OTF_CASE(1) BP5_OTF_CASE(2) BP5_OTF_CASE(3) BP5_OTF_CASE(4) BP5_OTF_CASE(5) BP5_OTF_CASE(6) BP5_OTF_CASE(7) BP5_OTF_CASE(8)
-#undef BP5_OTF_CASE
-    }
-  }
-  const int n3 = op->n * op->n * op->n;
+    op->cell_kernel = CellKernel::kOnTheFly;
+  else
+    op->cell_kernel = CellKernel::kOnTheFlyGeneral;
+  int cpt = 0;
+  const int rc = with_degree(op->p, [&](auto P) {
+    constexpr int p = decltype(P)::value;
+    cpt = op->cell_kernel == CellKernel::kOnTheFly          ? OtfTileCells<p>::value
+          : op->cell_kernel == CellKernel::kOnTheFlyGeneral ? OtfgTileCells<p>::value
+                                                            : TileCells<p>::value;
+    return BP5_OK;
+  });
+  if (rc != BP5_OK) return rc;
   op->cells_per_tile = cpt;
   operator_plan_tiles(op);
+  const int n3 = op->n * op->n * op->n;
   op->tile_doubles = ((int64_t)cpt * op->metric_planes * n3 + 1) & ~(int64_t)1;
-  // how the metric reaches the quadrature phase (ApplyCfg::MLOAD); BP5_MLOAD overrides for tuning runs
-  op->metric_path = 0;
-  // geometry on the fly on an undeformed (axis-parallel) mesh: one constant Jacobian, no coordinate gathers
-  const bool otf_affine = op->prob.geometry_mode == BP5_GEOM_ON_THE_FLY && op->prob.deformation == 0 &&
-                          op->prob.operator_kind == BP5_OP_POISSON;
-  if (otf_affine) { op->metric_path = 3; cpt = cells_per_tile_for(op->p); op->cells_per_tile = cpt; operator_plan_tiles(op); }
-#ifdef BP5_ENABLE_MLOAD
-  if (const char *mv = getenv("BP5_MLOAD")) op->metric_path = atoi(mv);
-#endif
-  BP5_REQUIRE(op->metric_path >= 0 && op->metric_path <= 3, "BP5_MLOAD must be 0, 1 or 2");
-  static const char *const kPath[4] = {"metric=tma-smem", "metric=ldg-regs", "metric=ldg-regs-ahead",
-                                       "geometry=on-the-fly(affine: constant Jacobian)"};
+  const char *quad = gll ? "gll-collocation" : "gauss", *kind = helm ? "helmholtz" : "poisson";
   char name[160];
-  snprintf(name, sizeof(name), "bp5_apply_kernel<p=%d,%s,%s,cells_per_tile=%d,%s>", op->p,
-           op->prob.quadrature == BP5_QUAD_GLL ? "gll-collocation" : "gauss",
-           op->prob.operator_kind == BP5_OP_HELMHOLTZ ? "helmholtz" : "poisson", cpt, kPath[op->metric_path]);
-  if (op->prob.geometry_mode == BP5_GEOM_ON_THE_FLY && !otf_affine) {
-    const bool special = !op->otf_general;
+  if (op->cell_kernel == CellKernel::kStored || op->cell_kernel == CellKernel::kAffine)
+    snprintf(name, sizeof(name), "bp5_apply_kernel<p=%d,%s,%s,cells_per_tile=%d,%s>", op->p, quad, kind, cpt,
+             op->cell_kernel == CellKernel::kAffine ? "geometry=on-the-fly(affine: constant Jacobian)" : "metric=tma-smem");
+  else
     snprintf(name, sizeof(name), "%s<p=%d,%s,%s,cells_per_tile=%d,geometry=on-the-fly>",
-             special ? "bp5_apply_otf_kernel" : "bp5_apply_otfg_kernel", op->p,
-             op->prob.quadrature == BP5_QUAD_GLL ? "gll-collocation" : "gauss",
-             op->prob.operator_kind == BP5_OP_HELMHOLTZ ? "helmholtz" : "poisson", cpt);
-  }
+             op->cell_kernel == CellKernel::kOnTheFly ? "bp5_apply_otf_kernel" : "bp5_apply_otfg_kernel", op->p, quad,
+             kind, cpt);
   op->kernel_name = name;
   return BP5_OK;
 }
 
-// mode: 0 dst += A src ; 1 overwrite cell-interior DoFs ; 2 = 1 + per-CTA partial sums of src . (A src)
-template <int P, int MLOAD>
-static int launch_pm(bp5_operator_t op, double *dst, const double *src, int mode, double *dp, int which) {
-  const bool gll = op->prob.quadrature == BP5_QUAD_GLL;
-  const bool helm = op->prob.operator_kind == BP5_OP_HELMHOLTZ;
-#define BP5_LAUNCH_MODE(M)                                                                                       \
-  (gll ? (helm ? launch<P, 1, 1, M, MLOAD>(op, dst, src, dp, which) : launch<P, 1, 0, M, MLOAD>(op, dst, src, dp, which))      \
-       : (helm ? launch<P, 0, 1, M, MLOAD>(op, dst, src, dp, which) : launch<P, 0, 0, M, MLOAD>(op, dst, src, dp, which)))
-  if constexpr (MLOAD == 0) {
-    if (op->hanging) return launch_hanging(op, dst, src, mode, dp, which);   // hanging-node constraints (apply_hang.cu)
-    if (mode >= 3) return launch_colored(op, dst, src, mode, dp, which);     // one colour, plain adds (apply_colored.cu)
-  }
-  if (mode == 2) return BP5_LAUNCH_MODE(2);
-  if (mode == 1) return BP5_LAUNCH_MODE(1);
-  return BP5_LAUNCH_MODE(0);
-#undef BP5_LAUNCH_MODE
-}
-
-// geometry on the fly, affine mesh (MLOAD = 3): Poisson only
-template <int P>
-static int launch_affine(bp5_operator_t op, double *dst, const double *src, int mode, double *dp, int which) {
-  const bool gll = op->prob.quadrature == BP5_QUAD_GLL;
-#define BP5_LAUNCH_AFF(M) (gll ? launch<P, 1, 0, M, 3>(op, dst, src, dp, which) : launch<P, 0, 0, M, 3>(op, dst, src, dp, which))
-  if (mode == 2) return BP5_LAUNCH_AFF(2);
-  if (mode == 1) return BP5_LAUNCH_AFF(1);
-  return BP5_LAUNCH_AFF(0);
-#undef BP5_LAUNCH_AFF
-}
-
-template <int P>
-static int launch_p(bp5_operator_t op, double *dst, const double *src, int mode, double *dp, int which) {
-  if (op->metric_path == 3) return launch_affine<P>(op, dst, src, mode, dp, which);
-#ifdef BP5_ENABLE_MLOAD   // tuning builds: metric straight to registers (measured slower, profiles/r1_v3_notes.md)
-  if (op->metric_path == 1) return launch_pm<P, 1>(op, dst, src, mode, dp, which);
-  if (op->metric_path == 2) return launch_pm<P, 2>(op, dst, src, mode, dp, which);
-#endif
-  return launch_pm<P, 0>(op, dst, src, mode, dp, which);
-}
-
+// mode: 0 dst += A src ; 1 overwrite cell-interior DoFs ; 2 = 1 + per-CTA partial sums of src . (A src) ;
+// 3..5 the same for one colour of the coloured cell order (plain adds)
 // overwrite_interior: dst's skeleton (shared DoFs, see zero_skeleton) must be
 // zero on entry, cell-interior DoFs are overwritten; otherwise dst += A src.
 // dot_partials != nullptr (needs overwrite_interior): the kernel also leaves op->apply_grid per-CTA parts of
 // src . (A src) there (see bp5_apply_kernel, OVERWRITE == 2).
-static int apply_dispatch(bp5_operator_t op, double *dst, const double *src, int mode, double *dot_partials, int which) {
-  if (op->prob.geometry_mode == BP5_GEOM_ON_THE_FLY && op->metric_path != 3)
-    return apply_cell_loop_otfg(op, dst, src, mode, dot_partials, which);
-  switch (op->p) {
-    case 1: return launch_p<1>(op, dst, src, mode, dot_partials, which);
-    case 2: return launch_p<2>(op, dst, src, mode, dot_partials, which);
-    case 3: return launch_p<3>(op, dst, src, mode, dot_partials, which);
-    case 4: return launch_p<4>(op, dst, src, mode, dot_partials, which);
-    case 5: return launch_p<5>(op, dst, src, mode, dot_partials, which);
-    case 6: return launch_p<6>(op, dst, src, mode, dot_partials, which);
-    case 7: return launch_p<7>(op, dst, src, mode, dot_partials, which);
-    case 8: return launch_p<8>(op, dst, src, mode, dot_partials, which);
+static int apply_dispatch(bp5_operator_t op, double *dst, const double *src, int mode, double *dp, int which) {
+  switch (op->cell_kernel) {
+    case CellKernel::kOnTheFly: return apply_cell_loop_otf(op, dst, src, mode, dp, which);
+    case CellKernel::kOnTheFlyGeneral: return apply_cell_loop_otfg(op, dst, src, mode, dp, which);
+    case CellKernel::kAffine:   // Poisson only
+      return with_degree(op->p, [&](auto P) {
+        return with_value<0, 1>(op->prob.quadrature == BP5_QUAD_GLL, [&](auto quad) {
+          return with_value<0, 1, 2>(mode, [&](auto m) {
+            return launch<P, quad, 0, m, true>(op, dst, src, dp, which);
+          });
+        });
+      });
+    case CellKernel::kStored:
+      if (op->hanging) return launch_hanging(op, dst, src, mode, dp, which);   // hanging-node constraints (apply_hang.cu)
+      if (mode >= 3) return launch_colored(op, dst, src, mode, dp, which);     // one colour, plain adds (apply_colored.cu)
+      return with_degree(op->p, [&](auto P) {
+        return with_quad_op(op, [&](auto quad, auto helm) {
+          return with_value<0, 1, 2>(mode, [&](auto m) { return launch<P, quad, helm, m>(op, dst, src, dp, which); });
+        });
+      });
   }
-  set_error("unsupported degree %d", op->p);
+  set_error("unknown cell kernel");
   return BP5_ERR_UNSUPPORTED;
 }
 

@@ -52,18 +52,14 @@ constexpr int kNoCell = INT_MIN;
 // e[m] = v[m] + v[N-1-m], o[m] = v[m] - v[N-1-m] (m < H = N/2) only the first H1 = ceil(N/2) rows are needed:
 //   pe = sum_m E[i][m] e[m] (+ C[i] v[H], N odd),  po = sum_m O[i][m] o[m],  out[i] = pe + po,  out[N-1-i] = S (pe - po)
 // -- about N^2/2 + 2N fp64 operations and half the matrix operands instead of N^2.  Packed as E | O | C.
-#ifndef BP5_EVENODD
-#define BP5_EVENODD 1
-#endif
 template <int N>
 struct EoShape {
   static constexpr int H = N / 2, H1 = (N + 1) / 2;
-  static constexpr int SIZE = BP5_EVENODD ? 2 * H1 * H + H1 : N * N;
+  static constexpr int SIZE = 2 * H1 * H + H1;
 };
 // host: M is N x N row-major
 template <int N>
 inline void pack_matrix(double *dst, const double *M) {
-  if (!BP5_EVENODD) { for (int i = 0; i < N * N; ++i) dst[i] = M[i]; return; }
   constexpr int H = EoShape<N>::H, H1 = EoShape<N>::H1;
   for (int i = 0; i < H1; ++i) {
     for (int m = 0; m < H; ++m) {
@@ -108,7 +104,7 @@ struct ApplyParams {
   const int *skip;        // optional device flag: non-zero => nothing to do (CG already converged)
   double *dot_partials;   // OVERWRITE == 2: [gridDim.x] per-CTA parts of src . (A src), summed by the CG dots kernel
   KernelTables<N> tab;
-  // MLOAD == 3 (geometry on the fly, affine mesh): G = w_q diag(aff) with aff = (hy hz / hx, hx hz / hy, hx hy / hz)
+  // AFFINE (geometry on the fly, affine mesh): G = w_q diag(aff) with aff = (hy hz / hx, hx hz / hy, hx hy / hz)
   // and the 1D quadrature weights wq.  (Behind `tab`: moving the tables in the parameter bank changes ptxas's
   // register allocation of the other kernels, p = 7 lost its third CTA per SM.)
   double aff[3];
@@ -163,15 +159,7 @@ __device__ __forceinline__ uint64_t make_evict_first_policy() {
   return pol;
 }
 
-// streaming 8-byte load for the metric when it goes straight to registers: read-only path,
-// no L1 allocation, L2 evict-first (every byte is used exactly once per operator application)
-__device__ __forceinline__ double ld_stream(const double *p, uint64_t policy) {
-  double v;
-  asm volatile("ld.global.nc.L1::no_allocate.L2::cache_hint.f64 %0, [%1], %2;" : "=d"(v) : "l"(p), "l"(policy));
-  return v;
-}
-
-// 8-byte asynchronous copy global -> shared (LDGSTS): the one-tile-ahead gather without registers (BP5_SMEM_PREFETCH)
+// 8-byte asynchronous copy global -> shared (LDGSTS): the one-tile-ahead gather without registers (kSmemPf)
 __device__ __forceinline__ void cp_async8(void *smem_dst, const void *gmem_src) {
   asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(smem_u32(smem_dst)), "l"(gmem_src) : "memory");
 }
@@ -205,19 +193,9 @@ __device__ __forceinline__ void gather_column(double (&u)[N], const double *__re
   for (int k = 0; k < N; ++k) u[k] = __ldg(src + idx[k]);
 }
 
-// Rows of the outer loop handled per (rolled) iteration: U independent DFMA
-// chains for latency hiding, with U*N matrix entries (2 uniform registers each)
-// live at a time -- must stay well inside the 63-entry uniform register file.
-// Measured (profiles/r1_v3_notes.md): n <= 8 full unroll everywhere.  n = 9 (81 matrix entries do not fit the
-// uniform register file): full unroll wins where the kernel still fits 4 CTAs/SM (<= 170 registers:
-// collocation without the fused dot product, Gauss with it), chunks of 3 rows elsewhere.
-#ifndef BP5_ROW_CHUNK
-#define BP5_ROW_CHUNK(N, QUAD, MODE) ((N) == 9 ? ((((QUAD) == 1 && (MODE) < 2) || ((QUAD) == 0 && (MODE) == 2)) ? 9 : 3) : (N))
-#endif
-
-// w = M v for a matrix with symmetry sign S (see EoShape); fully unrolled, result in registers
+// w = M v for a matrix with symmetry sign S (see EoShape); fully unrolled, result in registers (indexed statically)
 template <int N, int S>
-__device__ __forceinline__ void eo_matvec(double (&w)[N], const double *__restrict__ M, const double (&v)[N]) {
+__device__ __forceinline__ void contract_in_regs(double (&w)[N], const double *__restrict__ M, const double (&v)[N]) {
   constexpr int H = EoShape<N>::H, H1 = EoShape<N>::H1;
   const double *__restrict__ E = M, *__restrict__ O = M + H1 * H, *__restrict__ C = M + 2 * H1 * H;
   double e[H > 0 ? H : 1], o[H > 0 ? H : 1];
@@ -239,49 +217,14 @@ __device__ __forceinline__ void eo_matvec(double (&w)[N], const double *__restri
   }
 }
 
-// out[i*stride] = sum_m M[i][m] v[m].  Plain form (BP5_EVENODD == 0): outer loop ROLLED in chunks of U rows
-// (see header comment).
-template <int N, int U, int S>
+// out[i*stride] = sum_m M[i][m] v[m]
+template <int N, int S>
 __device__ __forceinline__ void contract_to_smem(double *out, int stride, const double *__restrict__ M,
                                                  const double (&v)[N]) {
-#if BP5_EVENODD
   double w[N];
-  eo_matvec<N, S>(w, M, v);
+  contract_in_regs<N, S>(w, M, v);
 #pragma unroll
   for (int i = 0; i < N; ++i) out[i * stride] = w[i];
-#else
-#pragma unroll 1
-  for (int i0 = 0; i0 < N; i0 += U) {
-    const double *row = M + i0 * N;
-    double s[U];
-#pragma unroll
-    for (int u = 0; u < U; ++u) s[u] = 0.0;
-#pragma unroll
-    for (int m = 0; m < N; ++m)
-#pragma unroll
-      for (int u = 0; u < U; ++u)
-        if (N % U == 0 || i0 + u < N) s[u] += row[u * N + m] * v[m];
-#pragma unroll
-    for (int u = 0; u < U; ++u)
-      if (N % U == 0 || i0 + u < N) out[(i0 + u) * stride] = s[u];
-  }
-#endif
-}
-
-// w[i] = sum_m M[i][m] v[m] in registers, fully unrolled (result indexed statically)
-template <int N, int S>
-__device__ __forceinline__ void contract_in_regs(double (&w)[N], const double *__restrict__ M, const double (&v)[N]) {
-#if BP5_EVENODD
-  eo_matvec<N, S>(w, M, v);
-#else
-#pragma unroll
-  for (int i = 0; i < N; ++i) {
-    double s = 0.0;
-#pragma unroll
-    for (int m = 0; m < N; ++m) s += M[i * N + m] * v[m];
-    w[i] = s;
-  }
-#endif
 }
 
 // ---- hanging-node constraints of the children of a locally refined mesh (HANG kernels only) ----------------------
@@ -339,21 +282,15 @@ __device__ __noinline__ void hang_exchange(unsigned int mask, bool active, int a
   if (T && z_line) line(hA, A2, M2);
 }
 
-// MLOAD: how the metric reaches the quadrature phase.
-//   0: one TMA bulk copy per tile into shared memory (mbarrier), read back with LDS;
-//   1: plain streaming loads into registers, issued at the start of the tile;
-//   2: the same, issued one tile ahead (right after the previous quadrature phase);
-//   3: no metric at all -- geometry on the fly on an AFFINE (axis-parallel) mesh: the Jacobian is one constant
-//      diagonal, G = w_q diag(hy hz / hx, hx hz / hy, hx hy / hz) is formed from kernel parameters.
-//      16 bytes per DoF of HBM traffic instead of 16 + 48 r: shared-memory-pipe / fp64 bound.
-// tuning builds may force a minimum number of resident CTAs per SM (-D'BP5_MIN_BLOCKS(P)=...');
-// by default ptxas's own heuristic is kept: an explicit minimum of 1 makes it spend ~50 more registers
-#ifdef BP5_MIN_BLOCKS
-#define BP5_LAUNCH_BOUNDS(NT, P) __launch_bounds__(NT, BP5_MIN_BLOCKS(P))
-#else
-#define BP5_LAUNCH_BOUNDS(NT, P) __launch_bounds__(NT)
-#endif
-template <int P, int CPT, int PLANES, int MLOAD = 0>
+// AFFINE: where G comes from.
+//   false: the stored metric, one TMA bulk copy per tile into shared memory (mbarrier), read back with LDS
+//          (measured faster than streaming it into registers, profiles/r1_v3_notes.md section 3);
+//   true:  no metric at all -- geometry on the fly on an AFFINE (axis-parallel) mesh: the Jacobian is one constant
+//          diagonal, G = w_q diag(hy hz / hx, hx hz / hy, hx hy / hz) is formed from kernel parameters.
+//          16 bytes per DoF of HBM traffic instead of 16 + 48 r: shared-memory-pipe / fp64 bound.
+// The kernels leave the minimum of resident CTAs per SM to ptxas's heuristic: an explicit minimum of 1 makes it spend
+// ~50 more registers.
+template <int P, int CPT, int PLANES, bool AFFINE = false>
 struct ApplyCfg {
   static constexpr int N = P + 1, N2 = N * N, N3 = N2 * N;
   using L = SmemLayout<N, CPT>;                            // per-array bank-conflict-minimising strides
@@ -362,14 +299,14 @@ struct ApplyCfg {
   static constexpr int METRIC_DOUBLES = (CPT * PLANES * N3 + 1) & ~1;  // per tile, padded to 16 bytes
   static constexpr uint32_t METRIC_BYTES = METRIC_DOUBLES * 8;
   static constexpr int WORK_DOUBLES = CPT * (2 * L::A_CS + L::B_CS);   // S0, S1 (layout A) and S2 (layout B)
-  static constexpr int STAGE_DOUBLES = MLOAD == 0 ? METRIC_DOUBLES : 0;   // shared-memory staging of the metric
+  static constexpr int STAGE_DOUBLES = AFFINE ? 0 : METRIC_DOUBLES;   // shared-memory staging of the metric
   // the mbarrier (8 bytes) goes into the padding word at the end of the first cell's S0 array when the layout
   // leaves one free, else behind the work arrays: at p = 7 those 16 bytes decide between 2 and 3 CTAs per SM
   // (3 x (76800 + 1024 reserved) = 233472 bytes = all of an SM's shared memory)
   static constexpr int A_LAST = (N - 1) * (L::A_S2 + L::A_S1 + 1);           // last used index of a layout-A array
   static constexpr bool BAR_IN_PAD = L::A_CS - 1 > A_LAST;
   static constexpr size_t SMEM_BYTES = (size_t)STAGE_DOUBLES * 8 + (size_t)WORK_DOUBLES * 8 + (BAR_IN_PAD ? 0 : 16);
-  static_assert(MLOAD != 3 || PLANES == 6, "the affine fast path is for the Poisson operator");
+  static_assert(!AFFINE || PLANES == 6, "the affine fast path is for the Poisson operator");
   static_assert(METRIC_BYTES % 16 == 0, "bulk copy size must be a multiple of 16 bytes");
 };
 
@@ -386,13 +323,12 @@ struct ApplyCfg {
 // HANG (locally refined meshes): 1 = the cells may carry hanging-node constraints (prm.cell_mask), resolved after the
 // gather and before the scatter -- one extra CTA-wide vote per tile, the exchange passes only in tiles that hold a masked
 // cell; 2 = no constrained cell in the tile range, only the per-cell stride classes of the refined numbering.
-template <int P, int QUAD, int HELM, int CPT, int OWMODE, int MLOAD = 0, int HANG = 0>
+template <int P, int QUAD, int HELM, int CPT, int OWMODE, bool AFFINE = false, int HANG = 0>
 __device__ __forceinline__ void bp5_apply_body(const ApplyParams<P + 1> &prm) {
   constexpr int OVERWRITE = OWMODE % 3;
   constexpr bool PLAIN_ADD = OWMODE >= 3;
-  using Cfg = ApplyCfg<P, CPT, 6 + HELM, MLOAD>;
+  using Cfg = ApplyCfg<P, CPT, 6 + HELM, AFFINE>;
   constexpr int N = Cfg::N, N2 = Cfg::N2, N3 = Cfg::N3, PLANES = 6 + HELM;
-  constexpr int RC = BP5_ROW_CHUNK(N, QUAD, OVERWRITE);     // rows per rolled iteration of a line contraction
   using L = typename Cfg::L;
   constexpr int A1 = L::A_S1, A2 = L::A_S2, B1 = L::B_S1, B2 = L::B_S2;
   extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -430,59 +366,36 @@ __device__ __forceinline__ void bp5_apply_body(const ApplyParams<P + 1> &prm) {
   const int *__restrict__ l2g_irr = prm.l2g_irr;
   const double *__restrict__ src = prm.src;
   double *__restrict__ dst = prm.dst;
-  const double *__restrict__ metric = prm.metric;
+  // prm.metric is read where the TMA copies are issued: a local copy of it is loaded once at the top of the kernel,
+  // and that changes ptxas's register allocation of the stored-metric kernels at most degrees
   uint64_t policy = 0;
-  if constexpr (MLOAD == 0) {
+  if constexpr (!AFFINE) {
     if (tid == 0) {
       mbar_init(bar, 1);
       fence_barrier_init();
       policy = make_evict_first_policy();
       if (tile0 < n_tiles) {
         mbar_expect_tx(bar, Cfg::METRIC_BYTES);
-        tma_load_1d(Gs, metric + tile0 * (long long)Cfg::METRIC_DOUBLES, Cfg::METRIC_BYTES, bar, policy);
+        tma_load_1d(Gs, prm.metric + tile0 * (long long)Cfg::METRIC_DOUBLES, Cfg::METRIC_BYTES, bar, policy);
       }
     }
     __syncthreads();
-  } else if constexpr (MLOAD != 3) {
-    policy = make_evict_first_policy();
   }
-  [[maybe_unused]] const double wab = MLOAD == 3 ? prm.wq[a] * prm.wq[b] : 0.0;
-  // this thread's column of the metric within a tile: [c][plane][k][b][a]
-  const int gcol = c * PLANES * N3 + b * N + a;
-  [[maybe_unused]] double greg[N][PLANES];
-  auto load_metric = [&](long long tile) {
-    const double *gp = metric + tile * (long long)Cfg::METRIC_DOUBLES + gcol;
-#pragma unroll
-    for (int k = 0; k < N; ++k)
-#pragma unroll
-      for (int pl = 0; pl < PLANES; ++pl) greg[k][pl] = ld_stream(gp + pl * N3 + k * N2, policy);
-  };
-  if constexpr (MLOAD == 2) {
-    if (active && tile0 < n_tiles) load_metric(tile0);
-  }
+  [[maybe_unused]] const double wab = AFFINE ? prm.wq[a] * prm.wq[b] : 0.0;
 
   // software pipeline of the gather: cell descriptors two tiles ahead, values one tile ahead
   int base_cur = (active && tile0 < n_tiles) ? __ldg(cell_base + tile0 * CPT + c) : kNoCell;
   int base_nxt = (active && tile0 + tstride < n_tiles) ? __ldg(cell_base + (tile0 + tstride) * CPT + c) : kNoCell;
-#ifndef BP5_PREFETCH_GATHER
-#ifdef BP5_NO_PREFETCH_P8      // tuning builds (scripts/build_variant.sh)
-#define BP5_PREFETCH_GATHER(P) ((P) != 8)
-#else
-#define BP5_PREFETCH_GATHER(P) 1
-#endif
-#endif
-  // BP5_SMEM_PREFETCH (collocation, conforming meshes): the next tile's columns are copied asynchronously (LDGSTS)
+  // kSmemPf (p = 8 collocation, conforming meshes): the next tile's columns are copied asynchronously (LDGSTS)
   // straight into S0 -- free from the end of the line phase (2) to the next tile's start -- instead of waiting in N
   // registers: the copy replaces the publishing stores, the home thread reads its column back for the z-derivative.
   // ptxas then needs 48-78 instead of 106-194 registers.  Measured at 148 M DoFs (profiles/r2_smem_prefetch_probe.log):
   // p = 8 cell loop 2.67 -> 2.33 ms (2 -> 4 CTAs/SM), merged CG 32.8 -> 34.8 GDoF*it/s; p = 5, 6 (shared memory
   // already limits the CTAs) 1-2 % slower -- the copy is in flight for 60 % of a tile instead of a whole one.
-  // Shipped for p = 8.  Value: bit m = used by the kernels of mode OVERWRITE == m.
-#ifndef BP5_SMEM_PREFETCH
-#define BP5_SMEM_PREFETCH(P) ((P) == 8 ? 7 : 0)
-#endif
-  constexpr bool kSmemPf = ((BP5_SMEM_PREFETCH(P) >> OVERWRITE) & 1) != 0 && QUAD == 1 && HANG == 0;
-  constexpr bool kPrefetch = BP5_PREFETCH_GATHER(P) != 0 && !kSmemPf;   // values of the next tile in registers one tile ahead
+  // Everywhere else the values of the next tile wait in registers (kPrefetch): without that prefetch p = 5, 6 gain a
+  // CTA per SM and still lose 9-13 % of the CG rate (profiles/r2_no_prefetch_p56_probe.log).
+  constexpr bool kSmemPf = P == 8 && QUAD == 1 && HANG == 0;
+  constexpr bool kPrefetch = !kSmemPf;   // values of the next tile in registers one tile ahead
   // HANG: the mask words travel with the cell descriptors (they select the strides of the gather)
   [[maybe_unused]] unsigned int w_cur = 0, w_nxt = 0;
   if constexpr (HANG) {
@@ -523,9 +436,6 @@ __device__ __forceinline__ void bp5_apply_body(const ApplyParams<P + 1> &prm) {
     if constexpr (HANG)
       w_n2 = (active && tile + 2 * tstride < n_tiles) ? __ldg(prm.cell_mask + (tile + 2 * tstride) * CPT + c) : 0u;
 
-    if constexpr (MLOAD == 1) {
-      if (active) load_metric(tile);
-    }
     [[maybe_unused]] unsigned int hmask = 0;
     [[maybe_unused]] bool tile_hangs = false;
     if constexpr (HANG == 1) {
@@ -554,10 +464,6 @@ __device__ __forceinline__ void bp5_apply_body(const ApplyParams<P + 1> &prm) {
 #pragma unroll
           for (int k = 0; k < N; ++k) s0[hA + k * A2] = u[k];
         }
-#ifdef BP5_GLL_DOUBLE_PUBLISH      // tuning builds: a second copy in layout B for the y-lines (no 2.8x conflict read of s0)
-#pragma unroll
-        for (int k = 0; k < N; ++k) s2[hB + k * B2] = u[k];
-#endif
         contract_in_regs<N, -1>(t, Dz, u);
         if constexpr (HELM) {
 #pragma unroll
@@ -570,14 +476,10 @@ __device__ __forceinline__ void bp5_apply_body(const ApplyParams<P + 1> &prm) {
         double v[N];
 #pragma unroll
         for (int i = 0; i < N; ++i) v[i] = s0[xA + i];
-        contract_to_smem<N, RC, -1>(s1 + xA, 1, Dx, v);
+        contract_to_smem<N, -1>(s1 + xA, 1, Dx, v);
 #pragma unroll
-#ifdef BP5_GLL_DOUBLE_PUBLISH
-        for (int j = 0; j < N; ++j) v[j] = s2[yB + j * B1];
-#else
         for (int j = 0; j < N; ++j) v[j] = s0[yA + j * A1];
-#endif
-        contract_to_smem<N, RC, -1>(s2 + yB, B1, Dy, v);
+        contract_to_smem<N, -1>(s2 + yB, B1, Dy, v);
       }
       __syncthreads();
       if constexpr (kSmemPf) {   // S0 is free until the next tile starts: fetch its columns behind the rest of this one
@@ -591,14 +493,14 @@ __device__ __forceinline__ void bp5_apply_body(const ApplyParams<P + 1> &prm) {
     } else {
       // ---------------- Gauss quadrature: interpolate to the q-points first
       // (1) home (i=a, j=b): z-interpolation
-      if (active) contract_to_smem<N, RC, 1>(s0 + hA, A2, Bz, u);
+      if (active) contract_to_smem<N, 1>(s0 + hA, A2, Bz, u);
       __syncthreads();
       // (2) x-line (j=a, qz=b): x-interpolation in place
       if (active) {
         double v[N];
 #pragma unroll
         for (int i = 0; i < N; ++i) v[i] = s0[xA + i];
-        contract_to_smem<N, RC, 1>(s0 + xA, 1, Bx, v);
+        contract_to_smem<N, 1>(s0 + xA, 1, Bx, v);
       }
       __syncthreads();
       // (3) y-line (qx=a, qz=b): y-interpolation (values at q-points), then d/dy
@@ -609,7 +511,7 @@ __device__ __forceinline__ void bp5_apply_body(const ApplyParams<P + 1> &prm) {
         contract_in_regs<N, 1>(w, By, v);
 #pragma unroll
         for (int q = 0; q < N; ++q) s0[yA + q * A1] = w[q];
-        contract_to_smem<N, RC, -1>(s2 + yB, B1, Dy, w);
+        contract_to_smem<N, -1>(s2 + yB, B1, Dy, w);
       }
       __syncthreads();
       // (4) x-line (qy=a, qz=b): d/dx ; home (qx=a, qy=b): d/dz in registers
@@ -617,7 +519,7 @@ __device__ __forceinline__ void bp5_apply_body(const ApplyParams<P + 1> &prm) {
         double v[N];
 #pragma unroll
         for (int i = 0; i < N; ++i) v[i] = s0[xA + i];
-        contract_to_smem<N, RC, -1>(s1 + xA, 1, Dx, v);
+        contract_to_smem<N, -1>(s1 + xA, 1, Dx, v);
 #pragma unroll
         for (int k = 0; k < N; ++k) v[k] = s0[hA + k * A2];
         contract_in_regs<N, -1>(t, Dz, v);
@@ -630,7 +532,7 @@ __device__ __forceinline__ void bp5_apply_body(const ApplyParams<P + 1> &prm) {
     }
 
     // ---------------- quadrature-point phase (home): g <- G g  (bp5/step-64.cu:160-188)
-    if constexpr (MLOAD == 0) {
+    if constexpr (!AFFINE) {
       mbar_wait(bar, parity);
       parity ^= 1;
     }
@@ -640,13 +542,11 @@ __device__ __forceinline__ void bp5_apply_body(const ApplyParams<P + 1> &prm) {
         const int q = (k * N + b) * N + a, wA = hA + k * A2, wB = hB + k * B2;
         const double ur = s1[wA], us = s2[wB], ut = t[k];
         double g0, g1, g2, g3, g4, g5;
-        if constexpr (MLOAD == 3) {
+        if constexpr (AFFINE) {
           const double w = wab * prm.wq[k];
           g0 = prm.aff[0] * w; g1 = prm.aff[1] * w; g2 = prm.aff[2] * w; g3 = g4 = g5 = 0.0;
-        } else if constexpr (MLOAD == 0) {
-          g0 = gm[q]; g1 = gm[N3 + q]; g2 = gm[2 * N3 + q]; g3 = gm[3 * N3 + q]; g4 = gm[4 * N3 + q]; g5 = gm[5 * N3 + q];
         } else {
-          g0 = greg[k][0]; g1 = greg[k][1]; g2 = greg[k][2]; g3 = greg[k][3]; g4 = greg[k][4]; g5 = greg[k][5];
+          g0 = gm[q]; g1 = gm[N3 + q]; g2 = gm[2 * N3 + q]; g3 = gm[3 * N3 + q]; g4 = gm[4 * N3 + q]; g5 = gm[5 * N3 + q];
         }
         const double vr = ur * g0 + us * g3 + ut * g4;
         const double vs = ur * g3 + us * g1 + ut * g5;
@@ -657,20 +557,18 @@ __device__ __forceinline__ void bp5_apply_body(const ApplyParams<P + 1> &prm) {
         if constexpr (OVERWRITE == 2) dot_acc += ur * vr + us * vs + ut * vt;
         if constexpr (HELM) {
           const double m_old = mv[k];
-          mv[k] = m_old * (MLOAD == 0 ? gm[6 * N3 + q] : greg[k][PLANES - 1]);
+          mv[k] = m_old * gm[6 * N3 + q];
           if constexpr (OVERWRITE == 2) dot_acc += m_old * mv[k];
         }
       }
     }
     __syncthreads();
-    if constexpr (MLOAD == 0) {
+    if constexpr (!AFFINE) {
       // the metric buffer is free: fetch the next tile's metric behind the remaining work
       if (tid == 0 && tile + tstride < n_tiles) {
         mbar_expect_tx(bar, Cfg::METRIC_BYTES);
-        tma_load_1d(Gs, metric + (tile + tstride) * (long long)Cfg::METRIC_DOUBLES, Cfg::METRIC_BYTES, bar, policy);
+        tma_load_1d(Gs, prm.metric + (tile + tstride) * (long long)Cfg::METRIC_DOUBLES, Cfg::METRIC_BYTES, bar, policy);
       }
-    } else if constexpr (MLOAD == 2) {
-      if (active && tile + tstride < n_tiles) load_metric(tile + tstride);
     }
 
     int idx[N];
@@ -684,10 +582,10 @@ __device__ __forceinline__ void bp5_apply_body(const ApplyParams<P + 1> &prm) {
         double v[N];
 #pragma unroll
         for (int i = 0; i < N; ++i) v[i] = s1[xA + i];
-        contract_to_smem<N, RC, -1>(s1 + xA, 1, DTx, v);
+        contract_to_smem<N, -1>(s1 + xA, 1, DTx, v);
 #pragma unroll
         for (int j = 0; j < N; ++j) v[j] = s2[yB + j * B1];
-        contract_to_smem<N, RC, -1>(s2 + yB, B1, DTy, v);
+        contract_to_smem<N, -1>(s2 + yB, B1, DTy, v);
       }
       __syncthreads();
       // (5) home: z-transpose in registers, sum the three directions, scatter
@@ -741,14 +639,14 @@ __device__ __forceinline__ void bp5_apply_body(const ApplyParams<P + 1> &prm) {
         double v[N];
 #pragma unroll
         for (int i = 0; i < N; ++i) v[i] = s1[xA + i];
-        contract_to_smem<N, RC, -1>(s1 + xA, 1, DTx, v);
+        contract_to_smem<N, -1>(s1 + xA, 1, DTx, v);
         if constexpr (HELM) {
           double o[N];
           contract_in_regs<N, -1>(o, DTz, t);
 #pragma unroll
           for (int k = 0; k < N; ++k) s0[hA + k * A2] = o[k] + mv[k];
         } else {
-          contract_to_smem<N, RC, -1>(s0 + hA, A2, DTz, t);
+          contract_to_smem<N, -1>(s0 + hA, A2, DTz, t);
         }
       }
       __syncthreads();
@@ -760,7 +658,7 @@ __device__ __forceinline__ void bp5_apply_body(const ApplyParams<P + 1> &prm) {
         contract_in_regs<N, -1>(y, DTy, v);
 #pragma unroll
         for (int q = 0; q < N; ++q) y[q] += s1[yA + q * A1] + s0[yA + q * A1];
-        contract_to_smem<N, RC, 1>(s0 + yA, A1, BTy, y);
+        contract_to_smem<N, 1>(s0 + yA, A1, BTy, y);
       }
       __syncthreads();
       // (7) x-line (j=a, qz=b): B^T along x in place
@@ -768,7 +666,7 @@ __device__ __forceinline__ void bp5_apply_body(const ApplyParams<P + 1> &prm) {
         double v[N];
 #pragma unroll
         for (int q = 0; q < N; ++q) v[q] = s0[xA + q];
-        contract_to_smem<N, RC, 1>(s0 + xA, 1, BTx, v);
+        contract_to_smem<N, 1>(s0 + xA, 1, BTx, v);
       }
       __syncthreads();
       // (8) home (i=a, j=b): B^T along z in registers, scatter
@@ -836,10 +734,10 @@ __device__ __forceinline__ void bp5_apply_body(const ApplyParams<P + 1> &prm) {
   }
 }
 
-template <int P, int QUAD, int HELM, int CPT, int OWMODE, int MLOAD = 0>
-__global__ void BP5_LAUNCH_BOUNDS((ApplyCfg<P, CPT, 6 + HELM, MLOAD>::NT), P)
+template <int P, int QUAD, int HELM, int CPT, int OWMODE, bool AFFINE = false>
+__global__ void __launch_bounds__(ApplyCfg<P, CPT, 6 + HELM, AFFINE>::NT)
     bp5_apply_kernel(const __grid_constant__ ApplyParams<P + 1> prm) {
-  bp5_apply_body<P, QUAD, HELM, CPT, OWMODE, MLOAD, 0>(prm);
+  bp5_apply_body<P, QUAD, HELM, CPT, OWMODE, AFFINE, 0>(prm);
 }
 
 // The kernels for locally refined meshes.  Their main loop is the conforming kernel's; the (not inlined) constraint
@@ -855,15 +753,15 @@ constexpr int hang_min_blocks() {
   return (P <= 6 ? 16 : 12) / warps;
 }
 template <int P, int QUAD, int HELM, int CPT, int OWMODE>
-__global__ void __launch_bounds__((ApplyCfg<P, CPT, 6 + HELM, 0>::NT), (hang_min_blocks<P, ApplyCfg<P, CPT, 6 + HELM, 0>::NT>()))
+__global__ void __launch_bounds__((ApplyCfg<P, CPT, 6 + HELM>::NT), (hang_min_blocks<P, ApplyCfg<P, CPT, 6 + HELM>::NT>()))
     bp5_apply_hang_kernel(const __grid_constant__ ApplyParams<P + 1> prm) {
-  bp5_apply_body<P, QUAD, HELM, CPT, OWMODE, 0, 1>(prm);
+  bp5_apply_body<P, QUAD, HELM, CPT, OWMODE, false, 1>(prm);
 }
 // the affine cells of a refined mesh: the conforming kernel plus the stride class per cell
 template <int P, int QUAD, int HELM, int CPT, int OWMODE>
-__global__ void BP5_LAUNCH_BOUNDS((ApplyCfg<P, CPT, 6 + HELM, 0>::NT), P)
+__global__ void __launch_bounds__(ApplyCfg<P, CPT, 6 + HELM>::NT)
     bp5_apply_strided_kernel(const __grid_constant__ ApplyParams<P + 1> prm) {
-  bp5_apply_body<P, QUAD, HELM, CPT, OWMODE, 0, 2>(prm);
+  bp5_apply_body<P, QUAD, HELM, CPT, OWMODE, false, 2>(prm);
 }
 
 }  // namespace bp5

@@ -4,29 +4,13 @@
 
 namespace bp5 {
 
-template <int P>
-static int launch_colored_p(bp5_operator_t op, double *dst, const double *src, int mode, double *dp, int which) {
-  const bool gll = op->prob.quadrature == BP5_QUAD_GLL;
-  const bool helm = op->prob.operator_kind == BP5_OP_HELMHOLTZ;
-  if (mode == 5) return BP5_LAUNCH_QH(P, 5, 0, 0);
-  if (mode == 4) return BP5_LAUNCH_QH(P, 4, 0, 0);
-  return BP5_LAUNCH_QH(P, 3, 0, 0);
-}
-
 int launch_colored(bp5_operator_t op, double *dst, const double *src, int mode, double *dp, int which) {
   BP5_REQUIRE(mode >= 3 && mode <= 5, "launch_colored: mode must be 3..5");
-  switch (op->p) {
-    case 1: return launch_colored_p<1>(op, dst, src, mode, dp, which);
-    case 2: return launch_colored_p<2>(op, dst, src, mode, dp, which);
-    case 3: return launch_colored_p<3>(op, dst, src, mode, dp, which);
-    case 4: return launch_colored_p<4>(op, dst, src, mode, dp, which);
-    case 5: return launch_colored_p<5>(op, dst, src, mode, dp, which);
-    case 6: return launch_colored_p<6>(op, dst, src, mode, dp, which);
-    case 7: return launch_colored_p<7>(op, dst, src, mode, dp, which);
-    case 8: return launch_colored_p<8>(op, dst, src, mode, dp, which);
-  }
-  set_error("unsupported degree %d", op->p);
-  return BP5_ERR_UNSUPPORTED;
+  return with_degree(op->p, [&](auto P) {
+    return with_quad_op(op, [&](auto quad, auto helm) {
+      return with_value<3, 4, 5>(mode, [&](auto m) { return launch<P, quad, helm, m>(op, dst, src, dp, which); });
+    });
+  });
 }
 
 }  // namespace bp5

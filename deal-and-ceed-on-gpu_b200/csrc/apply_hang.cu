@@ -4,35 +4,19 @@
 
 namespace bp5 {
 
-template <int P>
-static int launch_hanging_p(bp5_operator_t op, double *dst, const double *src, int mode, double *dp, int which) {
-  const bool gll = op->prob.quadrature == BP5_QUAD_GLL;
-  const bool helm = op->prob.operator_kind == BP5_OP_HELMHOLTZ;
+int launch_hanging(bp5_operator_t op, double *dst, const double *src, int mode, double *dp, int which) {
   BP5_REQUIRE(mode >= 0 && mode <= 2, "the coloured cell order is not available on locally refined meshes");
   BP5_REQUIRE(which == 1 || which == 2, "launch_hanging: one of the two tile groups at a time");
-  if (which == 1) {     // tiles [0, n_boundary_tiles): constrained cells and cells with an index table
-    if (mode == 2) return BP5_LAUNCH_QH(P, 2, 0, 1);
-    if (mode == 1) return BP5_LAUNCH_QH(P, 1, 0, 1);
-    return BP5_LAUNCH_QH(P, 0, 0, 1);
-  }
-  if (mode == 2) return BP5_LAUNCH_QH(P, 2, 0, 2);
-  if (mode == 1) return BP5_LAUNCH_QH(P, 1, 0, 2);
-  return BP5_LAUNCH_QH(P, 0, 0, 2);
-}
-
-int launch_hanging(bp5_operator_t op, double *dst, const double *src, int mode, double *dp, int which) {
-  switch (op->p) {
-    case 1: return launch_hanging_p<1>(op, dst, src, mode, dp, which);
-    case 2: return launch_hanging_p<2>(op, dst, src, mode, dp, which);
-    case 3: return launch_hanging_p<3>(op, dst, src, mode, dp, which);
-    case 4: return launch_hanging_p<4>(op, dst, src, mode, dp, which);
-    case 5: return launch_hanging_p<5>(op, dst, src, mode, dp, which);
-    case 6: return launch_hanging_p<6>(op, dst, src, mode, dp, which);
-    case 7: return launch_hanging_p<7>(op, dst, src, mode, dp, which);
-    case 8: return launch_hanging_p<8>(op, dst, src, mode, dp, which);
-  }
-  set_error("unsupported degree %d", op->p);
-  return BP5_ERR_UNSUPPORTED;
+  // which == 1: tiles [0, n_boundary_tiles), constrained cells and cells with an index table
+  return with_degree(op->p, [&](auto P) {
+    return with_quad_op(op, [&](auto quad, auto helm) {
+      return with_value<0, 1, 2>(mode, [&](auto m) {
+        return with_value<1, 2>(which, [&](auto hang) {
+          return launch<P, quad, helm, m, false, hang>(op, dst, src, dp, which);
+        });
+      });
+    });
+  });
 }
 
 }  // namespace bp5

@@ -1,79 +1,22 @@
 // Host side of the on-the-fly-geometry cell kernel (apply_otf.cuh): launch per degree and mode.
+#include "apply_launch.cuh"
 #include "apply_otf.cuh"
-#include "tile_cells.h"
 
 namespace bp5 {
 
-template <int P, int OVERWRITE>
-static int launch_otf(bp5_operator_t op, double *dst, const double *src, double *dot_partials, int which) {
-  constexpr int CPT = OtfTileCells<P>::value;
-  using Cfg = ApplyOtfCfg<P, CPT>;
-  constexpr int N = P + 1;
-  auto kernel = bp5_apply_otf_kernel<P, CPT, OVERWRITE>;
-  // per instantiation and per device: function attributes belong to the device's context, and the C ABI allows
-  // contexts on several devices in one process
-  static int blocks_per_sm_of[64] = {0};
-  int &blocks_per_sm = blocks_per_sm_of[op->ctx->device & 63];
-  if (blocks_per_sm == 0) {
-    BP5_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::SMEM_BYTES));
-    int nb = 0;
-    BP5_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, kernel, Cfg::NT, Cfg::SMEM_BYTES));
-    BP5_REQUIRE(nb > 0, "on-the-fly cell kernel does not fit on an SM");
-    blocks_per_sm = nb;
-  }
-  ApplyOtfParams<N> prm;
-  const long long n_local = op->n_owned + op->n_ghost;
-  prm.cx = op->coords; prm.cy = op->coords + n_local; prm.cz = op->coords + 2 * n_local;
-  prm.cell_base = op->cell_base; prm.l2g_irr = op->l2g_irr;
-  prm.src = src; prm.dst = dst;
-  prm.tile_begin = which == 2 ? op->n_boundary_tiles : 0;
-  prm.n_tiles = which == 1 ? op->n_boundary_tiles : op->n_tiles;
-  if (op->range_begin >= 0) { prm.tile_begin = op->range_begin; prm.n_tiles = op->range_end; }   // explicit tile range
-  prm.sy = op->od[0]; prm.sz = op->od[0] * op->od[1];
-  prm.skip = op->skip_flag;
-  prm.dot_partials = dot_partials;
-  if (prm.n_tiles <= prm.tile_begin) { op->apply_grid = 0; return BP5_OK; }
-  for (int q = 0; q < N; ++q) prm.wq[q] = op->tab.wq[q];
-  fill_kernel_tables<N>(prm.tab, op->tab.B, op->tab.Dt);
-  long long grid = (long long)blocks_per_sm * op->ctx->sm_count;
-  if (grid > prm.n_tiles - prm.tile_begin) grid = prm.n_tiles - prm.tile_begin;
-  if (grid < 1) grid = 1;
-  BP5_REQUIRE(grid <= kApplyPartialCap, "apply grid exceeds the partial-sum buffer");
-  op->apply_grid = (int)grid;
-  cudaEvent_t e0 = nullptr, e1 = nullptr;
-  if (op->profile) {
-    if (op->prof_used + 2 > op->prof_events.size())
-      for (int i = 0; i < 64; ++i) { cudaEvent_t e; BP5_CUDA(cudaEventCreate(&e)); op->prof_events.push_back(e); }
-    e0 = op->prof_events[op->prof_used++]; e1 = op->prof_events[op->prof_used++];
-    BP5_CUDA(cudaEventRecord(e0, op->ctx->stream));
-  }
-  kernel<<<(unsigned)grid, Cfg::NT, Cfg::SMEM_BYTES, op->ctx->stream>>>(prm);
-  BP5_CHECK_LAUNCH();
-  if (e1) BP5_CUDA(cudaEventRecord(e1, op->ctx->stream));
-  op->ctx->launches++;
-  return BP5_OK;
-}
-
-template <int P>
-static int launch_otf_p(bp5_operator_t op, double *dst, const double *src, int mode, double *dp, int which) {
-  if (mode == 2) return launch_otf<P, 2>(op, dst, src, dp, which);
-  if (mode == 1) return launch_otf<P, 1>(op, dst, src, dp, which);
-  return launch_otf<P, 0>(op, dst, src, dp, which);
-}
-
 int apply_cell_loop_otf(bp5_operator_t op, double *dst, const double *src, int mode, double *dot_partials, int which) {
-  switch (op->p) {
-    case 1: return launch_otf_p<1>(op, dst, src, mode, dot_partials, which);
-    case 2: return launch_otf_p<2>(op, dst, src, mode, dot_partials, which);
-    case 3: return launch_otf_p<3>(op, dst, src, mode, dot_partials, which);
-    case 4: return launch_otf_p<4>(op, dst, src, mode, dot_partials, which);
-    case 5: return launch_otf_p<5>(op, dst, src, mode, dot_partials, which);
-    case 6: return launch_otf_p<6>(op, dst, src, mode, dot_partials, which);
-    case 7: return launch_otf_p<7>(op, dst, src, mode, dot_partials, which);
-    case 8: return launch_otf_p<8>(op, dst, src, mode, dot_partials, which);
-  }
-  set_error("unsupported degree %d", op->p);
-  return BP5_ERR_UNSUPPORTED;
+  return with_degree(op->p, [&](auto P) {
+    return with_value<0, 1, 2>(mode, [&](auto m) {
+      constexpr int CPT = OtfTileCells<P>::value;
+      using Cfg = ApplyOtfCfg<P, CPT>;
+      ApplyOtfParams<P + 1> prm;
+      fill_common_params<P + 1>(prm, op, dst, src, dot_partials, which);
+      const long long n_local = op->n_owned + op->n_ghost;
+      prm.cx = op->coords; prm.cy = op->coords + n_local; prm.cz = op->coords + 2 * n_local;
+      return launch_cell_kernel<bp5_apply_otf_kernel<P, CPT, m>>(op, prm, Cfg::NT, Cfg::SMEM_BYTES,
+                                                                   cudaSharedmemCarveoutDefault);
+    });
+  });
 }
 
 }  // namespace bp5

@@ -54,7 +54,6 @@ __global__ void __launch_bounds__(ApplyOtfCfg<P, CPT>::NT)
   constexpr int N = Cfg::N, N2 = Cfg::N2;
   using L = typename Cfg::L;
   constexpr int A1 = L::A_S1, A2 = L::A_S2, B1 = L::B_S1, B2 = L::B_S2;
-  constexpr int RC = N == 9 ? 3 : N;
   extern __shared__ __align__(128) unsigned char smem_raw[];
   double *F = reinterpret_cast<double *>(smem_raw);      // [field][S0 | S1 | S2]
   constexpr int FS = Cfg::FIELD_DOUBLES, OS1 = CPT * L::A_CS, OS2 = 2 * CPT * L::A_CS;
@@ -104,7 +103,7 @@ __global__ void __launch_bounds__(ApplyOtfCfg<P, CPT>::NT)
 #pragma unroll
           for (int k = 0; k < N; ++k) s0[hA + k * A2] = col[k];
           if (f == 0) contract_in_regs<N, -1>(t, Dz, col);
-          else if constexpr (Cfg::ZSMEM) contract_to_smem<N, RC, -1>(Z + (f - 1) * ZS + cA + hA, A2, Dz, col);
+          else if constexpr (Cfg::ZSMEM) contract_to_smem<N, -1>(Z + (f - 1) * ZS + cA + hA, A2, Dz, col);
           else contract_in_regs<N, -1>(tc[f > 0 ? f - 1 : 0], Dz, col);
         }
       }
@@ -120,10 +119,10 @@ __global__ void __launch_bounds__(ApplyOtfCfg<P, CPT>::NT)
         double v[N];
 #pragma unroll
         for (int i = 0; i < N; ++i) v[i] = s0[xA + i];
-        contract_to_smem<N, RC, -1>(s1 + xA, 1, Dx, v);
+        contract_to_smem<N, -1>(s1 + xA, 1, Dx, v);
 #pragma unroll
         for (int j = 0; j < N; ++j) v[j] = s0[yA + j * A1];
-        contract_to_smem<N, RC, -1>(s2 + yB, B1, Dy, v);
+        contract_to_smem<N, -1>(s2 + yB, B1, Dy, v);
       };
       if constexpr (P == 5 || P == 7) {
 #pragma unroll
@@ -177,10 +176,10 @@ __global__ void __launch_bounds__(ApplyOtfCfg<P, CPT>::NT)
       double v[N];
 #pragma unroll
       for (int i = 0; i < N; ++i) v[i] = s1[xA + i];
-      contract_to_smem<N, RC, -1>(s1 + xA, 1, DTx, v);
+      contract_to_smem<N, -1>(s1 + xA, 1, DTx, v);
 #pragma unroll
       for (int j = 0; j < N; ++j) v[j] = s2[yB + j * B1];
-      contract_to_smem<N, RC, -1>(s2 + yB, B1, DTy, v);
+      contract_to_smem<N, -1>(s2 + yB, B1, DTy, v);
     }
     __syncthreads();
     // (5) home: z-transpose in registers, sum the three directions, scatter

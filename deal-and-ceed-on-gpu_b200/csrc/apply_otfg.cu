@@ -1,90 +1,25 @@
 // Host side of the general on-the-fly-geometry cell kernel (apply_otfg.cuh): launch per degree, quadrature,
-// operator and mode.  Gauss-Lobatto collocation + Poisson keeps its specialised kernel (apply_otf.cu).
+// operator and mode.  Gauss-Lobatto collocation + Poisson keeps its specialised kernel up to p = 4 (apply_otf.cu).
+#include "apply_launch.cuh"
 #include "apply_otfg.cuh"
-#include "tile_cells.h"
 
 namespace bp5 {
 
-template <int P, int QUAD, int HELM, int OVERWRITE>
-static int launch_otfg(bp5_operator_t op, double *dst, const double *src, double *dot_partials, int which) {
-  constexpr int CPT = OtfgTileCells<P>::value;
-  using Cfg = ApplyOtfgCfg<P, HELM, CPT, QUAD>;
-  constexpr int N = P + 1;
-  auto kernel = bp5_apply_otfg_kernel<P, QUAD, HELM, CPT, OVERWRITE>;
-  // per instantiation and per device (function attributes belong to the device's context)
-  static int blocks_per_sm_of[64] = {0};
-  int &blocks_per_sm = blocks_per_sm_of[op->ctx->device & 63];
-  if (blocks_per_sm == 0) {
-    BP5_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::SMEM_BYTES));
-    int nb = 0;
-    BP5_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, kernel, Cfg::NT, Cfg::SMEM_BYTES));
-    BP5_REQUIRE(nb > 0, "on-the-fly cell kernel does not fit on an SM");
-    blocks_per_sm = nb;
-  }
-  ApplyOtfgParams<N> prm;
-  const long long n_local = op->n_owned + op->n_ghost;
-  prm.cx = op->coords; prm.cy = op->coords + n_local; prm.cz = op->coords + 2 * n_local;
-  prm.cell_base = op->cell_base; prm.l2g_irr = op->l2g_irr;
-  prm.src = src; prm.dst = dst;
-  prm.tile_begin = which == 2 ? op->n_boundary_tiles : 0;
-  prm.n_tiles = which == 1 ? op->n_boundary_tiles : op->n_tiles;
-  if (op->range_begin >= 0) { prm.tile_begin = op->range_begin; prm.n_tiles = op->range_end; }   // explicit tile range
-  prm.sy = op->od[0]; prm.sz = op->od[0] * op->od[1];
-  prm.skip = op->skip_flag;
-  prm.dot_partials = dot_partials;
-  if (prm.n_tiles <= prm.tile_begin) { op->apply_grid = 0; return BP5_OK; }
-  for (int q = 0; q < N; ++q) prm.wq[q] = op->tab.wq[q];
-  fill_kernel_tables<N>(prm.tab, op->tab.B, op->tab.Dt);
-  long long grid = (long long)blocks_per_sm * op->ctx->sm_count;
-  if (grid > prm.n_tiles - prm.tile_begin) grid = prm.n_tiles - prm.tile_begin;
-  if (grid < 1) grid = 1;
-  BP5_REQUIRE(grid <= kApplyPartialCap, "apply grid exceeds the partial-sum buffer");
-  op->apply_grid = (int)grid;
-  cudaEvent_t e0 = nullptr, e1 = nullptr;
-  if (op->profile) {
-    if (op->prof_used + 2 > op->prof_events.size())
-      for (int i = 0; i < 64; ++i) { cudaEvent_t e; BP5_CUDA(cudaEventCreate(&e)); op->prof_events.push_back(e); }
-    e0 = op->prof_events[op->prof_used++]; e1 = op->prof_events[op->prof_used++];
-    BP5_CUDA(cudaEventRecord(e0, op->ctx->stream));
-  }
-  kernel<<<(unsigned)grid, Cfg::NT, Cfg::SMEM_BYTES, op->ctx->stream>>>(prm);
-  BP5_CHECK_LAUNCH();
-  if (e1) BP5_CUDA(cudaEventRecord(e1, op->ctx->stream));
-  op->ctx->launches++;
-  return BP5_OK;
-}
-
-template <int P, int QUAD, int HELM>
-static int launch_otfg_m(bp5_operator_t op, double *dst, const double *src, int mode, double *dp, int which) {
-  if (mode == 2) return launch_otfg<P, QUAD, HELM, 2>(op, dst, src, dp, which);
-  if (mode == 1) return launch_otfg<P, QUAD, HELM, 1>(op, dst, src, dp, which);
-  return launch_otfg<P, QUAD, HELM, 0>(op, dst, src, dp, which);
-}
-
-template <int P>
-static int launch_otfg_p(bp5_operator_t op, double *dst, const double *src, int mode, double *dp, int which) {
-  const bool gll = op->prob.quadrature == BP5_QUAD_GLL;
-  const bool helm = op->prob.operator_kind == BP5_OP_HELMHOLTZ;
-  if (!op->otf_general) return apply_cell_loop_otf(op, dst, src, mode, dp, which);
-  if (gll && !helm) return launch_otfg_m<P, 1, 0>(op, dst, src, mode, dp, which);
-  if (gll) return launch_otfg_m<P, 1, 1>(op, dst, src, mode, dp, which);
-  if (helm) return launch_otfg_m<P, 0, 1>(op, dst, src, mode, dp, which);
-  return launch_otfg_m<P, 0, 0>(op, dst, src, mode, dp, which);
-}
-
 int apply_cell_loop_otfg(bp5_operator_t op, double *dst, const double *src, int mode, double *dot_partials, int which) {
-  switch (op->p) {
-    case 1: return launch_otfg_p<1>(op, dst, src, mode, dot_partials, which);
-    case 2: return launch_otfg_p<2>(op, dst, src, mode, dot_partials, which);
-    case 3: return launch_otfg_p<3>(op, dst, src, mode, dot_partials, which);
-    case 4: return launch_otfg_p<4>(op, dst, src, mode, dot_partials, which);
-    case 5: return launch_otfg_p<5>(op, dst, src, mode, dot_partials, which);
-    case 6: return launch_otfg_p<6>(op, dst, src, mode, dot_partials, which);
-    case 7: return launch_otfg_p<7>(op, dst, src, mode, dot_partials, which);
-    case 8: return launch_otfg_p<8>(op, dst, src, mode, dot_partials, which);
-  }
-  set_error("unsupported degree %d", op->p);
-  return BP5_ERR_UNSUPPORTED;
+  return with_degree(op->p, [&](auto P) {
+    return with_quad_op(op, [&](auto quad, auto helm) {
+      return with_value<0, 1, 2>(mode, [&](auto m) {
+        constexpr int CPT = OtfgTileCells<P>::value;
+        using Cfg = ApplyOtfgCfg<P, helm, CPT>;
+        ApplyOtfgParams<P + 1> prm;
+        fill_common_params<P + 1>(prm, op, dst, src, dot_partials, which);
+        const long long n_local = op->n_owned + op->n_ghost;
+        prm.cx = op->coords; prm.cy = op->coords + n_local; prm.cz = op->coords + 2 * n_local;
+        return launch_cell_kernel<bp5_apply_otfg_kernel<P, quad, helm, CPT, m>>(op, prm, Cfg::NT, Cfg::SMEM_BYTES,
+                                                                                 cudaSharedmemCarveoutDefault);
+      });
+    });
+  });
 }
 
 }  // namespace bp5

@@ -35,18 +35,7 @@ struct ApplyOtfgParams {
   KernelTables<N> tab;
 };
 
-// tuning switches (profiles/r2_otf_general_tuning.log: both within +-5 %)
-// BP5_OTFG_PREFETCH: the gather of a field is issued one evaluation ahead (N more registers)
-#ifndef BP5_OTFG_PREFETCH
-#define BP5_OTFG_PREFETCH 1
-#endif
-// BP5_OTFG_DB (collocation): a second S0 array, so that the evaluation of a coordinate field needs ONE barrier
-// (publish | lines) instead of two -- the next field publishes into the other array while slow threads still read
-// this one
-#ifndef BP5_OTFG_DB
-#define BP5_OTFG_DB 0
-#endif
-template <int P, int HELM, int CPT, int QUAD = 0>
+template <int P, int HELM, int CPT>
 struct ApplyOtfgCfg {
   static constexpr int N = P + 1, N2 = N * N, N3 = N2 * N;
   using L = SmemLayout<N, CPT>;
@@ -58,27 +47,24 @@ struct ApplyOtfgCfg {
   static constexpr int JA_DOUBLES = 3 * CPT * L::A_CS, JB_DOUBLES = 3 * CPT * L::B_CS;
   static constexpr int JZ_PLANES = 3 + HELM;
   static constexpr int STAGE_DOUBLES = JA_DOUBLES + JB_DOUBLES + JZ_PLANES * CPT * N3;
-  static constexpr bool DB = QUAD == 1 && BP5_OTFG_DB != 0;
-  static constexpr int WORK_DOUBLES = CPT * ((DB ? 3 : 2) * L::A_CS + L::B_CS);    // S0 (x2), S1 (layout A), S2 (layout B)
+  static constexpr int WORK_DOUBLES = CPT * (2 * L::A_CS + L::B_CS);    // S0, S1 (layout A), S2 (layout B)
   static constexpr size_t SMEM_BYTES = ((size_t)STAGE_DOUBLES + WORK_DOUBLES) * 8;
 };
 
 // QUAD, HELM, OVERWRITE as in bp5_apply_kernel (0 add, 1 store cell-interior DoFs, 2 = 1 + partials of src.(A src))
 template <int P, int QUAD, int HELM, int CPT, int OVERWRITE>
-__global__ void __launch_bounds__(ApplyOtfgCfg<P, HELM, CPT, QUAD>::NT)
+__global__ void __launch_bounds__(ApplyOtfgCfg<P, HELM, CPT>::NT)
     bp5_apply_otfg_kernel(const __grid_constant__ ApplyOtfgParams<P + 1> prm) {
-  using Cfg = ApplyOtfgCfg<P, HELM, CPT, QUAD>;
-  constexpr bool DB = Cfg::DB;
+  using Cfg = ApplyOtfgCfg<P, HELM, CPT>;
   constexpr int N = Cfg::N, N2 = Cfg::N2, N3 = Cfg::N3;
   using L = typename Cfg::L;
   constexpr int A1 = L::A_S1, A2 = L::A_S2, B1 = L::B_S1, B2 = L::B_S2;
-  constexpr int RC = N == 9 ? 3 : N;
   extern __shared__ __align__(128) unsigned char smem_raw[];
   double *JA = reinterpret_cast<double *>(smem_raw);      // [3][CPT][A_CS]
   double *JB = JA + Cfg::JA_DOUBLES;                      // [3][CPT][B_CS]
   double *JZ = JB + Cfg::JB_DOUBLES;                      // [3 (+1)][CPT][N3]
   double *S0 = JA + Cfg::STAGE_DOUBLES;
-  double *S1 = S0 + (DB ? 2 : 1) * CPT * L::A_CS;
+  double *S1 = S0 + CPT * L::A_CS;
   double *S2 = S1 + CPT * L::A_CS;
 
   if (prm.skip != nullptr && *prm.skip != 0) return;
@@ -88,7 +74,6 @@ __global__ void __launch_bounds__(ApplyOtfgCfg<P, HELM, CPT, QUAD>::NT)
   const int r = tid % N2;
   const int a = r % N, b = r / N;
   double *s0 = S0 + c * L::A_CS, *s1 = S1 + c * L::A_CS, *s2 = S2 + c * L::B_CS;
-  [[maybe_unused]] double *s0b = s0 + CPT * L::A_CS;      // DB: the second S0 array (fields y and u)
   double *jz = JZ + c * N3 + b * N + a;                   // this thread's column: + field * CPT * N3 + k * N2
   const double *__restrict__ Bx = prm.tab.B[0], *__restrict__ By = prm.tab.B[1], *__restrict__ Bz = prm.tab.B[2];
   const double *__restrict__ BTx = prm.tab.BT[0], *__restrict__ BTy = prm.tab.BT[1], *__restrict__ BTz = prm.tab.BT[2];
@@ -111,11 +96,8 @@ __global__ void __launch_bounds__(ApplyOtfgCfg<P, HELM, CPT, QUAD>::NT)
 
   // values (mv, home column) and gradient (o1, layout A: d/dxi; o2, layout B: d/deta; t: d/dzeta in registers) of
   // one field at the quadrature points; the phases of bp5_apply_body.  Ends behind a barrier.
-  // sb: the S0 array of this evaluation; last_barrier: somebody reads o1 / o2 or rewrites sb right afterwards
-  auto evaluate = [&](const double (&u)[N], double (&t)[N], double (&mv)[N], double *o1, double *o2, double *sb,
-                      bool last_barrier) {
+  auto evaluate = [&](const double (&u)[N], double (&t)[N], double (&mv)[N], double *o1, double *o2) {
     if constexpr (QUAD == 1) {
-      double *s0 = sb;
       if (active) {
 #pragma unroll
         for (int k = 0; k < N; ++k) s0[hA + k * A2] = u[k];
@@ -128,20 +110,20 @@ __global__ void __launch_bounds__(ApplyOtfgCfg<P, HELM, CPT, QUAD>::NT)
         double v[N];
 #pragma unroll
         for (int i = 0; i < N; ++i) v[i] = s0[xA + i];
-        contract_to_smem<N, RC, -1>(o1 + xA, 1, Dx, v);
+        contract_to_smem<N, -1>(o1 + xA, 1, Dx, v);
 #pragma unroll
         for (int j = 0; j < N; ++j) v[j] = s0[yA + j * A1];
-        contract_to_smem<N, RC, -1>(o2 + yB, B1, Dy, v);
+        contract_to_smem<N, -1>(o2 + yB, B1, Dy, v);
       }
-      if (!DB || last_barrier) __syncthreads();
+      __syncthreads();
     } else {
-      if (active) contract_to_smem<N, RC, 1>(s0 + hA, A2, Bz, u);
+      if (active) contract_to_smem<N, 1>(s0 + hA, A2, Bz, u);
       __syncthreads();
       if (active) {
         double v[N];
 #pragma unroll
         for (int i = 0; i < N; ++i) v[i] = s0[xA + i];
-        contract_to_smem<N, RC, 1>(s0 + xA, 1, Bx, v);
+        contract_to_smem<N, 1>(s0 + xA, 1, Bx, v);
       }
       __syncthreads();
       if (active) {
@@ -151,14 +133,14 @@ __global__ void __launch_bounds__(ApplyOtfgCfg<P, HELM, CPT, QUAD>::NT)
         contract_in_regs<N, 1>(w, By, v);
 #pragma unroll
         for (int q = 0; q < N; ++q) s0[yA + q * A1] = w[q];
-        contract_to_smem<N, RC, -1>(o2 + yB, B1, Dy, w);
+        contract_to_smem<N, -1>(o2 + yB, B1, Dy, w);
       }
       __syncthreads();
       if (active) {
         double v[N];
 #pragma unroll
         for (int i = 0; i < N; ++i) v[i] = s0[xA + i];
-        contract_to_smem<N, RC, -1>(o1 + xA, 1, Dx, v);
+        contract_to_smem<N, -1>(o1 + xA, 1, Dx, v);
 #pragma unroll
         for (int k = 0; k < N; ++k) mv[k] = s0[hA + k * A2];
         contract_in_regs<N, -1>(t, Dz, mv);
@@ -168,8 +150,8 @@ __global__ void __launch_bounds__(ApplyOtfgCfg<P, HELM, CPT, QUAD>::NT)
   };
 
   // the gather of a field's columns is issued one evaluation ahead (the x coordinates of the next tile behind the
-  // solution field of this one): its L2 latency hides behind the contractions of the field before
-  constexpr bool PF = BP5_OTFG_PREFETCH != 0;
+  // solution field of this one): its L2 latency hides behind the contractions of the field before (N more registers;
+  // within +-5 % of gathering each field right before its evaluation, profiles/r2_otf_general_tuning.log)
   auto gather = [&](double (&v)[N], const double *__restrict__ fld, int bs) {
     int ix[N];
     column_indices<N>(ix, l2g_irr, bs, ab_off, ab_irr, sz);
@@ -179,16 +161,14 @@ __global__ void __launch_bounds__(ApplyOtfgCfg<P, HELM, CPT, QUAD>::NT)
   long long tile = prm.tile_begin + blockIdx.x;
   int base = (active && tile < n_tiles) ? __ldg(cell_base + tile * CPT + c) : kNoCell;
   double col[N];
-  if constexpr (PF) gather(col, prm.cx, base);
+  gather(col, prm.cx, base);
   for (; tile < n_tiles; tile += tstride) {
-    double t[N], mv[N];
-    [[maybe_unused]] double nxt[N];
+    double t[N], mv[N], nxt[N];
     // ---------------- geometry: Jacobian (and |x|^2) of the tile's cells at the quadrature points -> stage
 #pragma unroll 1
     for (int f = 0; f < 3; ++f) {
-      if constexpr (PF) gather(nxt, f == 0 ? prm.cy : f == 1 ? prm.cz : prm.src, base);
-      else gather(col, f == 0 ? prm.cx : f == 1 ? prm.cy : prm.cz, base);
-      evaluate(col, t, mv, JA + (f * CPT + c) * L::A_CS, JB + (f * CPT + c) * L::B_CS, (DB && (f & 1)) ? s0b : s0, false);
+      gather(nxt, f == 0 ? prm.cy : f == 1 ? prm.cz : prm.src, base);
+      evaluate(col, t, mv, JA + (f * CPT + c) * L::A_CS, JB + (f * CPT + c) * L::B_CS);
       if (active) {
         double *zp = jz + f * CPT * N3;
 #pragma unroll
@@ -200,17 +180,14 @@ __global__ void __launch_bounds__(ApplyOtfgCfg<P, HELM, CPT, QUAD>::NT)
           }
         }
       }
-      if constexpr (PF) {
 #pragma unroll
-        for (int k = 0; k < N; ++k) col[k] = nxt[k];
-      }
-      // no barrier: the next evaluation first writes S0 (DB: the other S0), which nobody reads any more
+      for (int k = 0; k < N; ++k) col[k] = nxt[k];
+      // no barrier: the next evaluation first writes S0, which nobody reads any more
     }
     // ---------------- the solution field
     const int base_n = (active && tile + tstride < n_tiles) ? __ldg(cell_base + (tile + tstride) * CPT + c) : kNoCell;
-    if constexpr (PF) gather(nxt, prm.cx, base_n);
-    else gather(col, prm.src, base);
-    evaluate(col, t, mv, s1, s2, DB ? s0b : s0, true);
+    gather(nxt, prm.cx, base_n);
+    evaluate(col, t, mv, s1, s2);
     // ---------------- quadrature-point phase (home): G from the staged Jacobian, g <- G g (+ mass term)
     if (active) {
 #pragma unroll
@@ -263,10 +240,10 @@ __global__ void __launch_bounds__(ApplyOtfgCfg<P, HELM, CPT, QUAD>::NT)
         double v[N];
 #pragma unroll
         for (int i = 0; i < N; ++i) v[i] = s1[xA + i];
-        contract_to_smem<N, RC, -1>(s1 + xA, 1, DTx, v);
+        contract_to_smem<N, -1>(s1 + xA, 1, DTx, v);
 #pragma unroll
         for (int j = 0; j < N; ++j) v[j] = s2[yB + j * B1];
-        contract_to_smem<N, RC, -1>(s2 + yB, B1, DTy, v);
+        contract_to_smem<N, -1>(s2 + yB, B1, DTy, v);
       }
       __syncthreads();
       if (do_scatter) {
@@ -286,7 +263,7 @@ __global__ void __launch_bounds__(ApplyOtfgCfg<P, HELM, CPT, QUAD>::NT)
         double v[N];
 #pragma unroll
         for (int i = 0; i < N; ++i) v[i] = s1[xA + i];
-        contract_to_smem<N, RC, -1>(s1 + xA, 1, DTx, v);
+        contract_to_smem<N, -1>(s1 + xA, 1, DTx, v);
         double o[N];
         contract_in_regs<N, -1>(o, DTz, t);
 #pragma unroll
@@ -300,14 +277,14 @@ __global__ void __launch_bounds__(ApplyOtfgCfg<P, HELM, CPT, QUAD>::NT)
         contract_in_regs<N, -1>(y, DTy, v);
 #pragma unroll
         for (int q = 0; q < N; ++q) y[q] += s1[yA + q * A1] + s0[yA + q * A1];
-        contract_to_smem<N, RC, 1>(s0 + yA, A1, BTy, y);
+        contract_to_smem<N, 1>(s0 + yA, A1, BTy, y);
       }
       __syncthreads();
       if (active) {
         double v[N];
 #pragma unroll
         for (int q = 0; q < N; ++q) v[q] = s0[xA + q];
-        contract_to_smem<N, RC, 1>(s0 + xA, 1, BTx, v);
+        contract_to_smem<N, 1>(s0 + xA, 1, BTx, v);
       }
       __syncthreads();
       if (do_scatter) {
@@ -326,10 +303,8 @@ __global__ void __launch_bounds__(ApplyOtfgCfg<P, HELM, CPT, QUAD>::NT)
     // no barrier here: the next tile first writes S0 -- the home columns (read last by their own threads) under
     // Gauss, an array nobody reads after the line phase under collocation
     base = base_n;
-    if constexpr (PF) {
 #pragma unroll
-      for (int k = 0; k < N; ++k) col[k] = nxt[k];
-    }
+    for (int k = 0; k < N; ++k) col[k] = nxt[k];
   }
   if constexpr (OVERWRITE == 2) {
     __syncthreads();

@@ -77,6 +77,14 @@ struct CgBuffers {
   double *hist;        // [hist_len] or nullptr
 };
 
+// The family of cell kernels an operator runs, chosen once by apply_choose
+enum class CellKernel {
+  kStored,             // stored metric (apply.cuh); coloured and hanging-node variants follow cell order and refinement
+  kAffine,             // geometry on the fly on an undeformed mesh: one constant Jacobian (apply.cuh, AFFINE)
+  kOnTheFly,           // geometry on the fly, collocation + Poisson, four fields at once (apply_otf.cuh)
+  kOnTheFlyGeneral,    // geometry on the fly, every quadrature / operator (apply_otfg.cuh)
+};
+
 // ---- handles ---------------------------------------------------------------
 }  // namespace bp5
 
@@ -113,7 +121,7 @@ struct bp5_operator_s {
   int64_t ghost_size[8] = {0};
   int cells_per_tile = 1;
   int apply_grid = 0;           // CTAs of the last cell-kernel launch (= number of fused-dot partial sums)
-  int metric_path = 0;          // ApplyCfg::MLOAD: 0 TMA -> shared memory, 1/2 streaming loads -> registers
+  bp5::CellKernel cell_kernel = bp5::CellKernel::kStored;
   int64_t n_tiles = 0;
   int64_t n_boundary_cells = 0;  // cells touching a lower ghost layer; they occupy tiles [0, n_boundary_tiles)
   int64_t n_boundary_tiles = 0;
@@ -133,8 +141,6 @@ struct bp5_operator_s {
   unsigned int *mfc_l2g[8] = {nullptr}, *mfc_constraint_mask[8] = {nullptr};
   double *mfc_inv_jacobian[8] = {nullptr}, *mfc_jxw[8] = {nullptr}, *mfc_q_points[8] = {nullptr};
   int64_t mfc_n_cells[8] = {0};
-  bool otf_general = false;     // BP5_GEOM_ON_THE_FLY on a deformed mesh: the general kernel (apply_otfg.cuh) instead of the
-                                // collocation + Poisson one (apply_otf.cuh)
   double *coords = nullptr;     // BP5_GEOM_ON_THE_FLY: nodal coordinates [3][n_owned + n_ghost] instead of the metric
   double *metric = nullptr;     // [tile][cpt][planes][n^3]; planes: 6 (Poisson) or 7 (Helmholtz: + a*JxW)
   int metric_planes = 6;
@@ -188,12 +194,12 @@ int operator_export_coefficients(bp5_operator_t op, double *host_out);
 int operator_export_coords(bp5_operator_t op, double *host_out);
 int operator_export_global_indices(bp5_operator_t op, int64_t *host_out);
 // apply.cu
-int apply_choose(bp5_operator_t op);                 // picks cells_per_tile + kernel name
+int apply_choose(bp5_operator_t op);                 // picks the kernel family, cells_per_tile, tile plan + kernel name
 // which: 0 all tiles, 1 boundary tiles only, 2 the others
 int apply_cell_loop(bp5_operator_t op, double *dst, const double *src, bool overwrite_interior,
                     double *dot_partials = nullptr, int which = 0);
+// the on-the-fly-geometry kernels (apply_otf.cu, apply_otfg.cu)
 int apply_cell_loop_otf(bp5_operator_t op, double *dst, const double *src, int mode, double *dot_partials, int which);
-// the general on-the-fly kernel (apply_otfg.cu): Gauss quadrature and / or Helmholtz; collocation + Poisson forwards to apply_cell_loop_otf
 int apply_cell_loop_otfg(bp5_operator_t op, double *dst, const double *src, int mode, double *dot_partials, int which);
 int apply_copy_constrained_dot(bp5_operator_t op, double *dst, const double *src, double *partials);
 int apply_zero_skeleton(bp5_operator_t op, double *dst);
