@@ -220,6 +220,10 @@ int bp5_operator_destroy(bp5_operator_t op) {
   cudaFree(op->coords);
   cudaFree(op->constrained);
   cudaFree(op->cg_scalars);
+  cudaFree(op->blk_desc);
+  cudaFree(op->blk_constrained);
+  bp5_vector_destroy(op->blk_x);
+  bp5_vector_destroy(op->blk_diag);
   for (cudaEvent_t e : op->prof_events) cudaEventDestroy(e);
   bp5_vector_destroy(op->g);
   bp5_vector_destroy(op->d);

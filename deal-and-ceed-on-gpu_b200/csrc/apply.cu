@@ -106,6 +106,12 @@ int apply_cell_loop(bp5_operator_t op, double *dst, const double *src, bool over
   return rc;
 }
 
+// the lexicographic in-loop kernels live in this file, the blocked ones in apply_blocked.cu
+int apply_cg_kernel_resources(bp5_operator_t op, bool blocked, int *ctas, size_t *local) {
+  if (blocked) return apply_blocked_kernel_resources(op, ctas, local);
+  return op_cg_kernel_resources<false>(op, ctas, local);
+}
+
 // "dst = 0" (bp5/step-64.cu:270-271) only has to reach the skeleton -- DoFs shared by several cells and the
 // ghosts; cell-interior DoFs are stored by the OVERWRITE kernel.  Measured (profiles/r1_v2_notes.md): zeroing
 // only the skeleton through a bit mask is SLOWER than a full memset (scattered partial-sector writes) and saves
@@ -151,9 +157,9 @@ __global__ void __launch_bounds__(256) copy_constrained_dot_kernel(const int *__
   }
 }
 
-int apply_copy_constrained_dot(bp5_operator_t op, double *dst, const double *src, double *partials) {
-  copy_constrained_dot_kernel<<<kConstrainedPartials, 256, 0, op->ctx->stream>>>(op->constrained, op->n_constrained, src,
-                                                                                dst, partials);
+int apply_copy_constrained_dot(bp5_operator_t op, const int *list, double *dst, const double *src, double *partials) {
+  copy_constrained_dot_kernel<<<kConstrainedPartials, 256, 0, op->ctx->stream>>>(list, op->n_constrained, src, dst,
+                                                                                partials);
   BP5_CHECK_LAUNCH();
   op->ctx->launches++;
   return BP5_OK;

@@ -116,6 +116,11 @@ struct ApplyParams {
   // cell_mask word, bits 8..10: stride class of an affine cell of a refined mesh (idx = base + i + j sy + k sz with
   // the class's strides: the numbering of a refined mesh is piecewise lexicographic)
   int hang_sy[8], hang_sz[8];
+  // BLK (the merged CG's blocked layout, BlockedLayout in common.h): per-cell starts [4][blk_stride] in class A
+  // (= cell_base), B, C and of the interior block; the offsets of a cell's upper y-face in class B and upper x-face in
+  // class C; the non-face y planes (class C's run length) and the size of one z-face plane of class A
+  const int *blk_desc;
+  int blk_stride, blk_up_b, blk_up_c, blk_ji, blk_plane;
 };
 
 __device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -184,13 +189,17 @@ __device__ __forceinline__ void column_indices(int (&idx)[N], const int *__restr
   }
 }
 
+// The same in the blocked layout: the column's ends lie on the cell's two z-faces (class A, one plane apart), the points
+// between them in one run of class B, C or the interior block (m0 + k m_str, m_off and m_str per thread).
 template <int N>
-__device__ __forceinline__ void gather_column(double (&u)[N], const double *__restrict__ src,
-                                              const int *__restrict__ l2g_irr, int base, int ab_off, int ab_irr, int sz) {
-  int idx[N];
-  column_indices<N>(idx, l2g_irr, base, ab_off, ab_irr, sz);
+__device__ __forceinline__ void column_indices_blk(int (&idx)[N], int base, int ab_off, int mbase, int m_off,
+                                                   int m_str, int plane) {
+  const bool cell = base != kNoCell;
+  const int a0 = cell ? base + ab_off : 0, m0 = cell ? mbase + m_off : 0, s = cell ? m_str : 0;
+  idx[0] = a0;
+  idx[N - 1] = cell ? a0 + plane : 0;
 #pragma unroll
-  for (int k = 0; k < N; ++k) u[k] = __ldg(src + idx[k]);
+  for (int k = 1; k < N - 1; ++k) idx[k] = m0 + k * s;
 }
 
 // w = M v for a matrix with symmetry sign S (see EoShape); fully unrolled, result in registers (indexed statically)
@@ -323,8 +332,11 @@ struct ApplyCfg {
 // HANG (locally refined meshes): 1 = the cells may carry hanging-node constraints (prm.cell_mask), resolved after the
 // gather and before the scatter -- one extra CTA-wide vote per tile, the exchange passes only in tiles that hold a masked
 // cell; 2 = no constrained cell in the tile range, only the per-cell stride classes of the refined numbering.
-template <int P, int QUAD, int HELM, int CPT, int OWMODE, bool AFFINE = false, int HANG = 0>
+// BLK: src and dst in the merged CG's blocked layout (conforming single block, default cell order); cell_base holds the
+// cells' class-A starts and prm.blk_desc the others.  Interior DoFs then share no sector with the skeleton.
+template <int P, int QUAD, int HELM, int CPT, int OWMODE, bool AFFINE = false, int HANG = 0, bool BLK = false>
 __device__ __forceinline__ void bp5_apply_body(const ApplyParams<P + 1> &prm) {
+  static_assert(!BLK || (HANG == 0 && OWMODE < 3), "the blocked layout is for the conforming, uncoloured kernels");
   constexpr int OVERWRITE = OWMODE % 3;
   constexpr bool PLAIN_ADD = OWMODE >= 3;
   using Cfg = ApplyCfg<P, CPT, 6 + HELM, AFFINE>;
@@ -404,12 +416,35 @@ __device__ __forceinline__ void bp5_apply_body(const ApplyParams<P + 1> &prm) {
   }
   auto off_of = [&](unsigned int w) { return HANG ? a + b * prm.hang_sy[(w >> 8) & 7u] : ab_off; };
   auto sz_of = [&](unsigned int w) { return HANG ? prm.hang_sz[(w >> 8) & 7u] : sz; };
+  // BLK: the class of this thread's column between the z-faces (1: B, on a y-face; 2: C, on an x-face only; 3: interior
+  // block), its offset in the cell's run and its stride; the cells' starts in that class travel with the descriptors
+  [[maybe_unused]] int m_cls = 0, m_off = 0, m_str = 0, m_cur = 0, m_nxt = 0;
+  if constexpr (BLK) {
+    const bool yface = b == 0 || b == P, xface = a == 0 || a == P;
+    m_cls = yface ? 1 : xface ? 2 : 3;
+    m_str = yface ? prm.sy : xface ? prm.blk_ji : (P - 1) * (P - 1);
+    m_off = (yface ? a + (b == P ? prm.blk_up_b : 0) : xface ? b - 1 + (a == P ? prm.blk_up_c : 0) : (b - 1) * (P - 1) + a - 1) -
+            m_str;
+    m_cur = (active && tile0 < n_tiles) ? __ldg(prm.blk_desc + m_cls * prm.blk_stride + tile0 * CPT + c) : 0;
+    m_nxt = (active && tile0 + tstride < n_tiles) ? __ldg(prm.blk_desc + m_cls * prm.blk_stride + (tile0 + tstride) * CPT + c)
+                                                  : 0;
+  }
+  auto indices = [&](int (&idx)[N], int base, unsigned int w, int mbase) {
+    if constexpr (BLK) column_indices_blk<N>(idx, base, ab_off, mbase, m_off, m_str, prm.blk_plane);
+    else column_indices<N>(idx, l2g_irr, base, off_of(w), ab_irr, sz_of(w));
+  };
+  auto gather = [&](double (&u)[N], int base, unsigned int w, int mbase) {
+    int idx[N];
+    indices(idx, base, w, mbase);
+#pragma unroll
+    for (int k = 0; k < N; ++k) u[k] = __ldg(src + idx[k]);
+  };
   [[maybe_unused]] double u_nxt[N];
-  if constexpr (kPrefetch) gather_column<N>(u_nxt, src, l2g_irr, base_cur, off_of(w_cur), ab_irr, sz_of(w_cur));
+  if constexpr (kPrefetch) gather(u_nxt, base_cur, w_cur, m_cur);
   if constexpr (kSmemPf) {
     if (active && tile0 < n_tiles) {
       int ix[N];
-      column_indices<N>(ix, l2g_irr, base_cur, off_of(w_cur), ab_irr, sz_of(w_cur));
+      indices(ix, base_cur, w_cur, m_cur);
 #pragma unroll
       for (int k = 0; k < N; ++k) cp_async8(s0 + hA + k * A2, src + ix[k]);
     }
@@ -427,14 +462,19 @@ __device__ __forceinline__ void bp5_apply_body(const ApplyParams<P + 1> &prm) {
 #pragma unroll
         for (int k = 0; k < N; ++k) u[k] = s0[hA + k * A2];
       }
-    } else if constexpr (!kPrefetch) gather_column<N>(u, src, l2g_irr, base_cur, off_of(w_cur), ab_irr, sz_of(w_cur));
+    } else if constexpr (!kPrefetch) gather(u, base_cur, w_cur, m_cur);
     // issue next tile's gather and the descriptor load of the tile after it
-    if constexpr (kPrefetch) gather_column<N>(u_nxt, src, l2g_irr, base_nxt, off_of(w_nxt), ab_irr, sz_of(w_nxt));
+    if constexpr (kPrefetch) gather(u_nxt, base_nxt, w_nxt, m_nxt);
     const int base_n2 =
         (active && tile + 2 * tstride < n_tiles) ? __ldg(cell_base + (tile + 2 * tstride) * CPT + c) : kNoCell;
     [[maybe_unused]] unsigned int w_n2 = 0;
     if constexpr (HANG)
       w_n2 = (active && tile + 2 * tstride < n_tiles) ? __ldg(prm.cell_mask + (tile + 2 * tstride) * CPT + c) : 0u;
+    [[maybe_unused]] int m_n2 = 0;
+    if constexpr (BLK)
+      m_n2 = (active && tile + 2 * tstride < n_tiles)
+                 ? __ldg(prm.blk_desc + m_cls * prm.blk_stride + (tile + 2 * tstride) * CPT + c)
+                 : 0;
 
     [[maybe_unused]] unsigned int hmask = 0;
     [[maybe_unused]] bool tile_hangs = false;
@@ -485,7 +525,7 @@ __device__ __forceinline__ void bp5_apply_body(const ApplyParams<P + 1> &prm) {
       if constexpr (kSmemPf) {   // S0 is free until the next tile starts: fetch its columns behind the rest of this one
         if (active && tile + tstride < n_tiles) {
           int ix[N];
-          column_indices<N>(ix, l2g_irr, base_nxt, off_of(w_nxt), ab_irr, sz_of(w_nxt));
+          indices(ix, base_nxt, w_nxt, m_nxt);
 #pragma unroll
           for (int k = 0; k < N; ++k) cp_async8(s0 + hA + k * A2, src + ix[k]);
         }
@@ -572,7 +612,7 @@ __device__ __forceinline__ void bp5_apply_body(const ApplyParams<P + 1> &prm) {
     }
 
     int idx[N];
-    column_indices<N>(idx, l2g_irr, base_cur, off_of(w_cur), ab_irr, sz_of(w_cur));
+    indices(idx, base_cur, w_cur, m_cur);
     const bool col_interior = OVERWRITE != 0 && a > 0 && a < P && b > 0 && b < P;
     const bool do_scatter = base_cur != kNoCell;
 
@@ -716,6 +756,7 @@ __device__ __forceinline__ void bp5_apply_body(const ApplyParams<P + 1> &prm) {
     base_cur = base_nxt;
     base_nxt = base_n2;
     if constexpr (HANG) { w_cur = w_nxt; w_nxt = w_n2; }
+    if constexpr (BLK) { m_cur = m_nxt; m_nxt = m_n2; }
   }
   if constexpr (OVERWRITE == 2) {
     // CTA-wide sum in a fixed order (warp shuffles, then warp 0 over the per-warp sums)
@@ -734,10 +775,10 @@ __device__ __forceinline__ void bp5_apply_body(const ApplyParams<P + 1> &prm) {
   }
 }
 
-template <int P, int QUAD, int HELM, int CPT, int OWMODE, bool AFFINE = false>
+template <int P, int QUAD, int HELM, int CPT, int OWMODE, bool AFFINE = false, bool BLK = false>
 __global__ void __launch_bounds__(ApplyCfg<P, CPT, 6 + HELM, AFFINE>::NT)
     bp5_apply_kernel(const __grid_constant__ ApplyParams<P + 1> prm) {
-  bp5_apply_body<P, QUAD, HELM, CPT, OWMODE, AFFINE, 0>(prm);
+  bp5_apply_body<P, QUAD, HELM, CPT, OWMODE, AFFINE, 0, BLK>(prm);
 }
 
 // The kernels for locally refined meshes.  Their main loop is the conforming kernel's; the (not inlined) constraint

@@ -88,8 +88,9 @@ static int launch_cell_kernel(bp5_operator_t op, const Params &prm, int nt, size
 }
 
 // One instantiation of the stored-metric kernel family (apply.cuh).  AFFINE: the constant-Jacobian kernel of an
-// undeformed mesh with geometry on the fly; HANG: the kernels of a locally refined mesh.
-template <int P, int QUAD, int HELM, int OWMODE, bool AFFINE = false, int HANG = 0>
+// undeformed mesh with geometry on the fly; HANG: the kernels of a locally refined mesh; BLK: the merged CG's blocked
+// layout (op->blk, set up by operator_setup_blocked).
+template <int P, int QUAD, int HELM, int OWMODE, bool AFFINE = false, int HANG = 0, bool BLK = false>
 static int launch(bp5_operator_t op, double *dst, const double *src, double *dot_partials, int which) {
   constexpr int CPT = TileCells<P>::value;
   using Cfg = ApplyCfg<P, CPT, 6 + HELM, AFFINE>;
@@ -98,7 +99,7 @@ static int launch(bp5_operator_t op, double *dst, const double *src, double *dot
   constexpr auto kernel = [] {
     if constexpr (HANG == 1) return bp5_apply_hang_kernel<P, QUAD, HELM, CPT, OWMODE>;
     else if constexpr (HANG == 2) return bp5_apply_strided_kernel<P, QUAD, HELM, CPT, OWMODE>;
-    else return bp5_apply_kernel<P, QUAD, HELM, CPT, OWMODE, AFFINE>;
+    else return bp5_apply_kernel<P, QUAD, HELM, CPT, OWMODE, AFFINE, BLK>;
   }();
   ApplyParams<N> prm;
   fill_common_params<N>(prm, op, dst, src, dot_partials, which);
@@ -110,9 +111,43 @@ static int launch(bp5_operator_t op, double *dst, const double *src, double *dot
   for (int cl = 0; cl < 8; ++cl) { prm.hang_sy[cl] = op->hang_sy[cl]; prm.hang_sz[cl] = op->hang_sz[cl]; }
   for (int sI = 0; sI < 2; ++sI)
     for (int i = 0; i < N * N; ++i) prm.hang[sI][i] = op->hanging_interp[sI][i];
+  prm.blk_desc = op->blk_desc;
+  prm.blk_stride = (int)(op->n_tiles * op->cells_per_tile);
+  prm.blk_up_b = op->blk.ki * op->blk.nx; prm.blk_up_c = op->blk.ki * op->blk.ji;
+  prm.blk_ji = op->blk.ji; prm.blk_plane = op->blk.nx * op->blk.ny;
+  if constexpr (BLK) prm.cell_base = op->blk_desc;
   // all of the L1/shared array as shared memory (the kernel's working set is its tiles; the gathers are
   // served by L2): with the default carve-out the p=6 kernel gets 2 instead of 3 CTAs per SM.
   return launch_cell_kernel<kernel>(op, prm, Cfg::NT, Cfg::SMEM_BYTES, cudaSharedmemCarveoutMaxShared);
+}
+
+// Resident CTAs per SM and local-memory bytes (spills, stack) of the in-loop kernel of the merged CG (OVERWRITE = 2), in
+// the lexicographic (BLK = false) or the blocked layout, with the launch attributes `launch` sets.
+template <int P, int QUAD, int HELM, bool AFFINE, bool BLK>
+static int cg_kernel_resources(int *ctas, size_t *local) {
+  constexpr int CPT = TileCells<P>::value;
+  using Cfg = ApplyCfg<P, CPT, 6 + HELM, AFFINE>;
+  constexpr auto kernel = bp5_apply_kernel<P, QUAD, HELM, CPT, 2, AFFINE, BLK>;
+  BP5_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::SMEM_BYTES));
+  BP5_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+  BP5_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(ctas, kernel, Cfg::NT, Cfg::SMEM_BYTES));
+  cudaFuncAttributes fa;
+  BP5_CUDA(cudaFuncGetAttributes(&fa, kernel));
+  *local = fa.localSizeBytes;
+  return BP5_OK;
+}
+
+// the same for op's kernel family (stored metric or affine) and degree, quadrature and operator
+template <bool BLK>
+static int op_cg_kernel_resources(bp5_operator_t op, int *ctas, size_t *local) {
+  if (op->cell_kernel == CellKernel::kAffine)
+    return with_degree(op->p, [&](auto P) {
+      return with_value<0, 1>(op->prob.quadrature == BP5_QUAD_GLL,
+                              [&](auto quad) { return cg_kernel_resources<P, quad, 0, true, BLK>(ctas, local); });
+    });
+  return with_degree(op->p, [&](auto P) {
+    return with_quad_op(op, [&](auto quad, auto helm) { return cg_kernel_resources<P, quad, helm, false, BLK>(ctas, local); });
+  });
 }
 
 // defined in apply_colored.cu / apply_hang.cu

@@ -80,13 +80,14 @@ __device__ __forceinline__ void block_sum_k(double (&v)[K], double *sh /*[K*32]*
 // MODE 0: update_a0 (solver.h:48-72)  1: update_a<false> (:74-104)  3: update_a1 (:106-140)
 // Fused here: r.r (and r.Dr) of the residual this kernel WRITES -- two of the seven sums of update_b
 // (solver.h:142-311) -- as per-block partials rr[block][2], so the dots pass does not have to form them.
+// zero_from: start of the skeleton in the blocked layout (the cell kernel stores the interior blocks), else 0
 template <int MODE, bool DIAG>
 __global__ void __launch_bounds__(256) cg_update_kernel(const CgState *__restrict__ st, double *__restrict__ p,
                                                         double *__restrict__ r, double *__restrict__ v,
                                                         double *__restrict__ x, const double *__restrict__ diag,
-                                                        double *__restrict__ rr, long long n) {
-  // "v = 0" (solver.h:69,101,137).  (Restricting it to the skeleton was measured slower: scattered
-  // partial-sector writes, and L2 fills the sectors anyway.)
+                                                        double *__restrict__ rr, long long n, long long zero_from) {
+  // "v = 0" (solver.h:69,101,137).  (Restricting it to the skeleton of the lexicographic layout was measured slower:
+  // scattered partial-sector writes, and L2 fills the sectors anyway.  The blocked layout's skeleton is one range.)
   if (st->state != 0) return;
   __shared__ double sh[2 * 32];
   const double alpha = st->alpha, beta = st->beta;
@@ -107,7 +108,7 @@ __global__ void __launch_bounds__(256) cg_update_kernel(const CgState *__restric
       r[i] = r_new;
       p[i] = beta * p_old - dg * r_new;
     }
-    v[i] = 0.0;
+    if (i >= zero_from) v[i] = 0.0;
     s[0] += r_new * r_new;
     if (DIAG) s[1] += r_new * dg * r_new;
   }
@@ -333,22 +334,24 @@ int cg_status(int state, int it, double res) {
 // 1) update region (solver.h:413-448) of iteration `cur` (1-based), with the parity-correct x update, plus r.r and
 //    r.Dr of the new residual as per-block partials in cb.rr.  The kernel zeroes h; its ghost entries receive the
 //    contributions for the neighbouring owners, so they start at zero too.
+//    zero_from: first entry of h to zero (the skeleton of the blocked layout; 0 otherwise).
 template <int MODE>
 static void launch_update(unsigned grid, cudaStream_t s, const CgBuffers &cb, double *p, double *r, double *v,
-                          double *x, const double *diag, long long n) {
-  if (diag) cg_update_kernel<MODE, true><<<grid, 256, 0, s>>>(cb.st, p, r, v, x, diag, cb.rr, n);
-  else cg_update_kernel<MODE, false><<<grid, 256, 0, s>>>(cb.st, p, r, v, x, diag, cb.rr, n);
+                          double *x, const double *diag, long long n, long long zero_from) {
+  if (diag) cg_update_kernel<MODE, true><<<grid, 256, 0, s>>>(cb.st, p, r, v, x, diag, cb.rr, n, zero_from);
+  else cg_update_kernel<MODE, false><<<grid, 256, 0, s>>>(cb.st, p, r, v, x, diag, cb.rr, n, zero_from);
 }
 
-static int enqueue_update(bp5_operator_t op, const CgBuffers &cb, int cur, double *x, const double *diag) {
+static int enqueue_update(bp5_operator_t op, const CgBuffers &cb, int cur, double *x, const double *diag,
+                          long long zero_from = 0) {
   const long long n = op->n_owned;
   const unsigned grid = stream_grid(n, op->ctx->sm_count);
   BP5_REQUIRE(grid <= (unsigned)kUpdatePartialCap, "update grid exceeds the partial-sum buffer");
   cudaStream_t s = op->ctx->stream;
   double *g = op->g->d, *d = op->d->d, *h = op->h->d;
-  if (cur == 1) launch_update<0>(grid, s, cb, d, g, h, x, diag, n);
-  else if (cur % 2 == 0) launch_update<1>(grid, s, cb, d, g, h, x, diag, n);
-  else launch_update<3>(grid, s, cb, d, g, h, x, diag, n);
+  if (cur == 1) launch_update<0>(grid, s, cb, d, g, h, x, diag, n, zero_from);
+  else if (cur % 2 == 0) launch_update<1>(grid, s, cb, d, g, h, x, diag, n, zero_from);
+  else launch_update<3>(grid, s, cb, d, g, h, x, diag, n, zero_from);
   BP5_CHECK_LAUNCH();
   op->ctx->launches++;
   if (op->n_ghost) BP5_CUDA(cudaMemsetAsync(h + n, 0, sizeof(double) * op->n_ghost, s));
@@ -357,10 +360,11 @@ static int enqueue_update(bp5_operator_t op, const CgBuffers &cb, int cur, doubl
 
 // 2) h = A d: apply_cell_loop(op, h, d, true, cb.ph) with do_zero_out = false (solver.h:475; h's skeleton is zeroed by
 //    the update kernel, its cell-interior entries are overwritten by the cell kernel) leaves d.h as per-CTA partials.
-// 3) Dirichlet copy h_c = d_c, with its correction of d.h after the cell loop's n_ph partials.
-static int enqueue_constrained(bp5_operator_t op, const CgBuffers &cb, int n_ph) {
+// 3) Dirichlet copy h_c = d_c, with its correction of d.h after the cell loop's n_ph partials.  list: the Dirichlet
+//    DoFs in the layout of the work vectors.
+static int enqueue_constrained(bp5_operator_t op, const CgBuffers &cb, int n_ph, const int *list = nullptr) {
   if (op->n_constrained == 0) return BP5_OK;
-  return apply_copy_constrained_dot(op, op->h->d, op->d->d, cb.ph + n_ph);
+  return apply_copy_constrained_dot(op, list ? list : op->constrained, op->h->d, op->d->d, cb.ph + n_ph);
 }
 
 // partials of d.h once the Dirichlet copy has followed a cell loop that left n_ph
@@ -467,12 +471,13 @@ static int run_iterations(bp5_operator_t op, CgState *st, int max_its, Enqueue e
 
 // End of cg_solve() / cg_solve_peer() after run_iterations() returned rc: the owed x update (x == nullptr: none, as
 // in the standard CG), the final state, history[1..], last_step / last_value and the return code.  peer: the
-// transport's error word is checked before the state is decoded.
+// transport's error word is checked before the state is decoded.  x_user: x is the blocked layout's copy of x_user.
 static int finish_solve(bp5_operator_t op, const CgBuffers &cb, int rc, double *x, const double *diag, bool peer,
-                        double *history, int hist_len, int *last_step, double *last_value) {
+                        double *history, int hist_len, int *last_step, double *last_value, double *x_user = nullptr) {
   cudaStream_t s = op->ctx->stream;
   op->skip_flag = nullptr;
   if (rc == BP5_OK && x) rc = enqueue_finish(op, cb.st, x, diag);
+  if (rc == BP5_OK && x_user) rc = vec_blocked_permute(op->ctx, op->blk, x_user, x, 1.0, /*to_blocked=*/false);
   CgState fin{};
   cudaError_t e1 = cudaMemcpyAsync(&fin, cb.st, sizeof(CgState), cudaMemcpyDeviceToHost, s);
   cudaError_t e2 = cudaStreamSynchronize(s);
@@ -492,6 +497,15 @@ static int finish_solve(bp5_operator_t op, const CgBuffers &cb, int rc, double *
   return cg_status(fin.state, fin.it, fin.res);
 }
 
+// *v exists or could be allocated (an out-of-memory error is cleared, not reported)
+static bool spare_vector(bp5_operator_t op, bp5_vector_t *v) {
+  if (*v) return true;
+  if (bp5_vector_create(op->ctx, op->n_owned, 0, v) == BP5_OK) return true;
+  cudaGetLastError();
+  set_error("%s", "");
+  return false;
+}
+
 int cg_solve(bp5_operator_t op, bp5_vector_t x, bp5_vector_t b, bp5_vector_t diagv, int variant, int control,
              double tol, int max_its, int *last_step, double *last_value, double *history, int history_len) {
   bp5_context_t ctx = op->ctx;
@@ -508,17 +522,36 @@ int cg_solve(bp5_operator_t op, bp5_vector_t x, bp5_vector_t b, bp5_vector_t dia
   if ((rc = cg_buffers(op, hist_len, &cb))) return rc;
   CgState *st = cb.st;
   double *g = op->g->d, *d = op->d->d, *h = op->h->d;
+  // The merged CG on one conforming block runs in the blocked layout (BlockedLayout, common.h): its work vectors, the
+  // diagonal and a copy of x; x and b stay in the user's layout, permuted once at the start and x once at the end.
+  bool blk = variant == BP5_CG_MERGED && operator_blocked_supported(op);
+  if (blk && (rc = operator_setup_blocked(op))) return rc;
+  // the copies of x and of the diagonal are the solver's to spare: where they do not fit next to the user's data, the
+  // solve keeps the lexicographic layout instead of failing
+  blk = blk && spare_vector(op, &op->blk_x) && (!diag || spare_vector(op, &op->blk_diag));
+  double *xs = blk ? op->blk_x->d : x->d;
 
   // g = A x - b, or -b if x == 0 (solver.h:375-381)
   int x_zero = 0;
   if ((rc = vec_all_zero(ctx, x->d, n, &x_zero))) return rc;
   if (!x_zero) {
-    if ((rc = apply_zero_skeleton(op, g))) return rc;
-    if ((rc = apply_cell_loop(op, g, x->d, true))) return rc;
-    if ((rc = apply_copy_constrained(op, g, x->d))) return rc;
-    if ((rc = vec_axpy(ctx, g, 1.0, -1.0, b->d, n, 0))) return rc;
+    double *t = blk ? h : g;   // blocked: formed in the user's layout in h, then permuted into g
+    if ((rc = apply_zero_skeleton(op, t))) return rc;
+    if ((rc = apply_cell_loop(op, t, x->d, true))) return rc;
+    if ((rc = apply_copy_constrained(op, t, x->d))) return rc;
+    if ((rc = vec_axpy(ctx, t, 1.0, -1.0, b->d, n, 0))) return rc;
+    if (blk && ((rc = vec_blocked_permute(ctx, op->blk, g, h, 1.0, true)) ||
+                (rc = vec_blocked_permute(ctx, op->blk, xs, x->d, 1.0, true))))
+      return rc;
+  } else if (blk) {
+    if ((rc = vec_blocked_permute(ctx, op->blk, g, b->d, -1.0, true))) return rc;
+    BP5_CUDA(cudaMemsetAsync(xs, 0, sizeof(double) * n, s));
   } else if ((rc = vec_axpy(ctx, g, 0.0, -1.0, b->d, n, 1)))
     return rc;
+  if (blk && diag) {
+    if ((rc = vec_blocked_permute(ctx, op->blk, op->blk_diag->d, diag, 1.0, true))) return rc;
+    diag = op->blk_diag->d;
+  }
   double gg = 0.0;
   if ((rc = vec_dot(ctx, g, g, n, &gg))) return rc;
   double res = std::sqrt(gg);
@@ -549,9 +582,9 @@ int cg_solve(bp5_operator_t op, bp5_vector_t x, bp5_vector_t b, bp5_vector_t dia
   auto enqueue = [&](int cur) -> int {
     int rc;
     if (variant == BP5_CG_MERGED) {   // the stepwise sequence, with the scalar recurrences fused into the dots kernel
-      if ((rc = enqueue_update(op, cb, cur, x->d, diag))) return rc;
-      if ((rc = apply_cell_loop(op, h, d, true, cb.ph))) return rc;
-      if ((rc = enqueue_constrained(op, cb, op->apply_grid))) return rc;
+      if ((rc = enqueue_update(op, cb, cur, xs, diag, blk ? op->blk.sa : 0))) return rc;
+      if ((rc = blk ? apply_cell_loop_blocked(op, h, d, cb.ph) : apply_cell_loop(op, h, d, true, cb.ph))) return rc;
+      if ((rc = enqueue_constrained(op, cb, op->apply_grid, blk ? op->blk_constrained : nullptr))) return rc;
       return enqueue_dots<true>(op, cb, diag, /*lean=*/true, nullptr, ph_count(op, op->apply_grid), (int)grid);
     }
     if ((rc = apply_zero_skeleton(op, h))) return rc;
@@ -569,8 +602,8 @@ int cg_solve(bp5_operator_t op, bp5_vector_t x, bp5_vector_t b, bp5_vector_t dia
     return BP5_OK;
   };
   rc = run_iterations(op, st, max_its, enqueue);
-  return finish_solve(op, cb, rc, variant == BP5_CG_MERGED ? x->d : nullptr, diag, /*peer=*/false, history, hist_len,
-                      last_step, last_value);
+  return finish_solve(op, cb, rc, variant == BP5_CG_MERGED ? xs : nullptr, diag, /*peer=*/false, history, hist_len,
+                      last_step, last_value, blk ? x->d : nullptr);
 }
 
 // ------------------------------------------------------------------------

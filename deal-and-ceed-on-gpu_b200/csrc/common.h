@@ -77,6 +77,20 @@ struct CgBuffers {
   double *hist;        // [hist_len] or nullptr
 };
 
+// The merged CG's blocked DoF layout on one conforming block (blocked.cuh): [interior blocks | skeleton].  Each cell's
+// (p-1)^3 interior DoFs are one contiguous block, in the cell processing order; the skeleton (lattice points with a
+// coordinate on a cell face) comes in three classes, each affine in a cell's local coordinates:
+//   A  points on z-face planes, lexicographic (x, y, plane);
+//   B  points on y-face planes and not on a z-face plane, (x, non-face z, plane);
+//   C  points on x-face planes only, (non-face y, non-face z, plane) -- y fastest, so a cell's x-face is read in runs.
+// Interior DoFs are touched by one cell only and share no 32-byte sector with the skeleton's atomics.
+struct BlockedLayout {
+  int p = 0, nc[3] = {0, 0, 0};   // degree, cells per direction
+  int nx = 0, ny = 0;             // lattice points in x and y (p nc + 1)
+  int ki = 0, ji = 0;             // non-face lattice planes in z and in y: nc (p - 1)
+  long long sa = 0, sb = 0, sc = 0, n = 0;   // starts of the classes A, B, C (sa = number of interior DoFs); size
+};
+
 // The family of cell kernels an operator runs, chosen once by apply_choose
 enum class CellKernel {
   kStored,             // stored metric (apply.cuh); coloured and hanging-node variants follow cell order and refinement
@@ -167,6 +181,14 @@ struct bp5_operator_s {
   bp5::CgBuffers cg_buf{};      // stepwise CG: cg_scalars as laid out by cg_step_begin
   bool cg_ph_valid = false;     // stepwise CG: the cell kernel left d.h partials for the next dots step
   int cg_update_grid = 0;       // stepwise CG: blocks (= r.r partials) of the last update step
+  // merged CG in the blocked layout (operator_setup_blocked, built by the first solve that takes it)
+  bp5::BlockedLayout blk{};
+  int *blk_desc = nullptr;        // [4][n_tiles * cells_per_tile] per-cell starts in class A, B, C and of the interior
+                                  // block; class A: kNoCell for tile padding
+  int *blk_constrained = nullptr; // the Dirichlet list in the blocked layout
+  bp5_vector_t blk_x = nullptr, blk_diag = nullptr;   // the solution and the diagonal in the blocked layout
+  int blk_fits = -1;              // the blocked in-loop kernel keeps the lexicographic one's CTAs/SM, no more spill
+                                  // (1 / 0, -1: not yet asked)
   // live per-launch timing of the cell kernel (bench.py roofline): events around every launch
   bool profile = false;
   std::vector<cudaEvent_t> prof_events;   // start/stop pairs
@@ -190,6 +212,8 @@ int operator_l2_norm_sqr(bp5_operator_t op, const double *u_dev, double *out);
 int operator_generic_data(bp5_operator_t op);
 int operator_generic_data_colored(bp5_operator_t op);
 int operator_diagonal(bp5_operator_t op, double *diag_dev, bool invert);
+bool operator_blocked_supported(bp5_operator_t op);         // the merged CG can run in the blocked layout
+int operator_setup_blocked(bp5_operator_t op);            // op->blk, blk_desc, blk_constrained (first call only)
 int operator_export_coefficients(bp5_operator_t op, double *host_out);
 int operator_export_coords(bp5_operator_t op, double *host_out);
 int operator_export_global_indices(bp5_operator_t op, int64_t *host_out);
@@ -201,7 +225,13 @@ int apply_cell_loop(bp5_operator_t op, double *dst, const double *src, bool over
 // the on-the-fly-geometry kernels (apply_otf.cu, apply_otfg.cu)
 int apply_cell_loop_otf(bp5_operator_t op, double *dst, const double *src, int mode, double *dot_partials, int which);
 int apply_cell_loop_otfg(bp5_operator_t op, double *dst, const double *src, int mode, double *dot_partials, int which);
-int apply_copy_constrained_dot(bp5_operator_t op, double *dst, const double *src, double *partials);
+// the merged CG's cell loop in the blocked layout (apply_blocked.cu): overwrite interior, per-CTA partials of src.(A src)
+int apply_cell_loop_blocked(bp5_operator_t op, double *dst, const double *src, double *dot_partials);
+int apply_blocked_kernel_resources(bp5_operator_t op, int *ctas, size_t *local);
+// resident CTAs per SM and local-memory bytes of the merged CG's in-loop cell kernel, lexicographic or blocked
+int apply_cg_kernel_resources(bp5_operator_t op, bool blocked, int *ctas, size_t *local);
+// list: the Dirichlet DoFs in the layout of dst and src (op->constrained or op->blk_constrained)
+int apply_copy_constrained_dot(bp5_operator_t op, const int *list, double *dst, const double *src, double *partials);
 int apply_zero_skeleton(bp5_operator_t op, double *dst);
 int apply_copy_constrained(bp5_operator_t op, double *dst, const double *src);
 // vector.cu
@@ -209,6 +239,9 @@ int vec_fill(bp5_context_t ctx, double *d, int64_t n, double v);
 int vec_axpy(bp5_context_t ctx, double *y, double s, double a, const double *x, int64_t n, int mode);
 int vec_dot(bp5_context_t ctx, const double *x, const double *y, int64_t n, double *out);
 int vec_all_zero(bp5_context_t ctx, const double *x, int64_t n, int *out);
+// to_blocked: dst[blocked(t)] = scale * src[t]; otherwise dst[t] = scale * src[blocked(t)] (t lexicographic)
+int vec_blocked_permute(bp5_context_t ctx, const BlockedLayout &L, double *dst, const double *src, double scale,
+                        bool to_blocked);
 // halo.cu
 int halo_info(bp5_operator_t op, int64_t *send_count, int64_t *send_offset, int64_t *recv_count, int64_t *recv_offset);
 int halo_pack(bp5_operator_t op, const double *vec, double *sendbuf);

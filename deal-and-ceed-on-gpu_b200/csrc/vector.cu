@@ -4,7 +4,7 @@
 // (bp5/solver.h:375-382,511 ; bp5/step-64.cu:445,449,467).
 // Reductions are deterministic: fixed grid, per-block partials, one block sums
 // them in a fixed order.
-#include "common.h"
+#include "blocked.cuh"
 
 namespace bp5 {
 
@@ -24,6 +24,21 @@ __global__ void axpy_kernel(double *__restrict__ y, double s, double a, const do
     else if (MODE == 1) y[i] = a * x[i];
     else if (MODE == 2) y[i] = s * y[i] + a * x[i];
     else y[i] *= x[i];
+  }
+}
+
+// the merged CG's layout change at the start and the end of a solve, one pass each
+template <bool TO_BLOCKED>
+__global__ void blocked_permute_kernel(BlockedLayout L, double *__restrict__ dst, const double *__restrict__ src,
+                                       double scale) {
+  const long long plane = (long long)L.nx * L.ny;
+  for (long long t = blockIdx.x * (long long)blockDim.x + threadIdx.x; t < L.n; t += (long long)gridDim.x * blockDim.x) {
+    const int k = (int)(t / plane);
+    const int j = (int)((t - k * plane) / L.nx);
+    const int i = (int)(t - k * plane - (long long)j * L.nx);
+    const long long bi = blocked_index(L, i, j, k);
+    if (TO_BLOCKED) dst[bi] = scale * src[t];
+    else dst[t] = scale * src[bi];
   }
 }
 
@@ -98,6 +113,17 @@ int vec_axpy(bp5_context_t ctx, double *y, double s, double a, const double *x, 
   else if (mode == 1) axpy_kernel<1><<<g, 256, 0, ctx->stream>>>(y, s, a, x, n);
   else if (mode == 2) axpy_kernel<2><<<g, 256, 0, ctx->stream>>>(y, s, a, x, n);
   else axpy_kernel<3><<<g, 256, 0, ctx->stream>>>(y, s, a, x, n);
+  BP5_CHECK_LAUNCH();
+  ctx->launches++;
+  return BP5_OK;
+}
+
+int vec_blocked_permute(bp5_context_t ctx, const BlockedLayout &L, double *dst, const double *src, double scale,
+                        bool to_blocked) {
+  if (L.n == 0) return BP5_OK;
+  const unsigned g = grid_for(L.n, 256, 148 * 16);
+  if (to_blocked) blocked_permute_kernel<true><<<g, 256, 0, ctx->stream>>>(L, dst, src, scale);
+  else blocked_permute_kernel<false><<<g, 256, 0, ctx->stream>>>(L, dst, src, scale);
   BP5_CHECK_LAUNCH();
   ctx->launches++;
   return BP5_OK;
